@@ -10,6 +10,7 @@ stream), so the hot-pair list a fold leaves behind is a prediction for the next 
 not a replay of it; the very first window (no history) is timed separately.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5]
+                  [--dump-outputs DIR]
 
 Configs are BASELINE.json's (index into `configs`):
   2 (default, the one `metric` is quoted on at N=1): 10k services / 100M events per GPU per step
@@ -77,6 +78,8 @@ def parse_args():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-gnn", action="store_true", help="skip the separate GNN-update timing (config 2)")
     ap.add_argument("--no-verify", action="store_true", help="skip the in-run parity check against the oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's edges (and GNN scores) to DIR/*.npy, see dump_outputs()")
     return ap.parse_args()
 
 
@@ -91,6 +94,8 @@ def resolve(args, world):
         n_rank = c["events"] // world
     steps = args.steps if args.steps is not None else c["steps"]
     warmup = args.warmup if args.warmup is not None else c["warmup"]
+    if steps < 1:
+        raise SystemExit("bench.py: --steps must be at least 1")
     return c, S, n_rank, steps, max(3, warmup)
 
 
@@ -296,8 +301,12 @@ def main():
 
     # ---- inputs resident in HBM before the timed region: R distinct windows, rotated
     free_b, _ = torch.cuda.mem_get_info()
-    R = args.windows or max(1, min(4 if args.config == 2 else 10 if args.config == 5 else 2,
-                                   int((free_b * 0.55) // (N * 32))))
+    R_want = args.windows or (4 if args.config == 2 else 10 if args.config == 5 else 2)
+    R = args.windows or max(1, min(R_want, int((free_b * 0.55) // (N * 32))))
+    if args.dump_outputs and R != R_want:
+        # the last timed step reads window (warmup + steps - 1) % R: with fewer windows it would be other events
+        raise SystemExit(f"bench.py: --dump-outputs needs all {R_want} input windows resident, only {R} fit "
+                         f"in free device memory")
     d_win, first = [], 0
     for k in range(R):
         d = h.dev_alloc(N * 32)
@@ -348,18 +357,23 @@ def main():
     sampler.mark()
     ev = [[torch.cuda.Event(enable_timing=True) for _ in range(4)] for _ in range(steps)]
     t_all0, t_all1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    p_scores = None
     t_all0.record(stream)
     for k in range(steps):
         ev[k][0].record(stream)
         h.submit_device(d_win[(warmup + k) % R], N)
         ev[k][1].record(stream)
-        _, n_edges = h.flush_device()
+        p_edges, n_edges = h.flush_device()
         ev[k][2].record(stream)
         if with_gnn:
-            gnn_score_device(h)
+            p_scores, n_scores = gnn_score_device(h)
         ev[k][3].record(stream)
     t_all1.record(stream)
     barrier()
+    if args.dump_outputs and rank == 0:   # before verify_window: the next flush overwrites these device buffers
+        if with_gnn and n_scores != n_edges:
+            raise SystemExit(f"bench.py: {n_scores} GNN scores for {n_edges} edges")
+        dump_outputs(args.dump_outputs, abi, torch, p_edges, n_edges, p_scores)
     total_ms = t_all0.elapsed_time(t_all1)
     ingest_ms = float(np.mean([e[0].elapsed_time(e[1]) for e in ev]))
     flush_ms = float(np.mean([e[1].elapsed_time(e[2]) for e in ev]))
@@ -471,6 +485,36 @@ def gnn_score_device(h):
     p, n_out = C.c_void_p(), C.c_size_t(0)
     h._ck(h.L.alz_gnn_score_device(h.h, C.byref(p), C.byref(n_out)), "alz_gnn_score_device")
     return p.value, n_out.value
+
+
+DUMP_MAX_EDGES = 1 << 16          # 71 float64 columns a row: at most 37 MB of edges.npy
+
+
+def dump_outputs(out_dir, abi, torch, p_edges, n_edges, p_scores):
+    """Writes what alz_window_flush_device (and alz_gnn_score_device) returned in the last timed step, so that two
+    builds can be compared output for output. One float64 row per edge: from_type, to_type, from, to, count, err5xx,
+    lat_sum_ns, hist[0..63], in the library's canonical edge order; above DUMP_MAX_EDGES edges a fixed seeded sample
+    of the rows (edge_rows.npy says which). scores.npy: float32 GNN scores of the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = int(n_edges)
+    rows = np.arange(n)
+    if n > DUMP_MAX_EDGES:
+        rows = np.sort(np.random.default_rng(SEED).choice(n, DUMP_MAX_EDGES, replace=False))
+    idx = torch.from_numpy(rows).to("cuda")
+    words = abi.EDGE_OUT.itemsize // 4
+    e = np.zeros(0, dtype=abi.EDGE_OUT)
+    if n:
+        sel = dev_view(torch, p_edges, n * words).view(n, words).index_select(0, idx)
+        e = sel.cpu().numpy().view(abi.EDGE_OUT).reshape(-1)
+    cols = [e[f].astype(np.float64)[:, None] for f in ("from_type", "to_type", "from", "to", "count", "err5xx",
+                                                        "lat_sum_ns")]
+    np.save(os.path.join(out_dir, "edges.npy"), np.hstack(cols + [e["hist"].astype(np.float64)]))
+    np.save(os.path.join(out_dir, "edge_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "n_edges.npy"), np.array([n], dtype=np.float64))
+    if p_scores is not None:
+        s = dev_view(torch, p_scores, n).index_select(0, idx).cpu().numpy().view(np.float32) if n else \
+            np.zeros(0, dtype=np.float32)
+        np.save(os.path.join(out_dir, "scores.npy"), s)
 
 
 def verify_window(h, capi, abi, topo, d_ev, N, S, world, rank, dist, torch):

@@ -1,14 +1,15 @@
 #!/usr/bin/env python
 """Extracts the input vector of the reference's own KAT TestSocketLine (aggregator/sock_line_test.go:11-349:
 the tsList literal and the queried timestamp) into tests/golden/sockline_kat.json, so that the KAT can be
-replayed in full (all timestamps) where /root/reference does not exist (the GPU box). Run in the build
-container:  python tests/golden/make_sockline_fixture.py
+replayed in full (all timestamps) without a checkout of the reference. Run with the path of a getanteon/alaz
+checkout at 828b997f:  python tests/golden/make_sockline_fixture.py <alaz checkout>
 """
 import json
 import os
 import re
+import sys
 
-REF = "/root/reference/aggregator/sock_line_test.go"
+REF = os.path.join(sys.argv[1], "aggregator", "sock_line_test.go")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "sockline_kat.json")
 
 src = open(REF).read()
