@@ -26,14 +26,11 @@
 
 using namespace alz;
 
-#define CK(expr)                                                                       \
-  do {                                                                                 \
-    cudaError_t _e = (expr);                                                           \
-    if (_e != cudaSuccess) {                                                           \
-      h->last_err = std::string(#expr) + ": " + cudaGetErrorString(_e);                \
-      return ALZ_E_CUDA;                                                               \
-    }                                                                                  \
-  } while (0)
+int alz_error(alz_handle* h, int rc, const char* what, const char* why) {
+  std::lock_guard<std::mutex> g(h->err_mu);
+  h->last_err = what ? std::string(what) + ": " + why : std::string(why);
+  return rc;
+}
 
 static uint32_t next_pow2(uint64_t x) {
   uint64_t p = 1;
@@ -60,45 +57,41 @@ static int alloc_table(alz_handle* h, AccTable* t, uint32_t max_rows, uint32_t* 
   const uint32_t dict_cap = next_pow2(2ull * max_rows);
   t->dict_mask = dict_cap - 1;
   const size_t rows = (size_t)max_rows + kPairKinds;
-  CK(cudaMalloc(&t->dict, (size_t)dict_cap * sizeof(DictEnt)));
-  CK(cudaMalloc(&t->row_key, rows * 8));
+  Owned& m = h->mem;
+  CK(m.dev(&t->dict, (size_t)dict_cap * sizeof(DictEnt)));
+  CK(m.dev(&t->row_key, rows * 8));
   if (!pair_table) {
-    CK(cudaMalloc(&t->lat_sum, rows * 8));
-    CK(cudaMalloc(&t->err5xx, rows * 8));
-    CK(cudaMalloc(&t->count, rows * 8));
-    CK(cudaMalloc(&t->hist, rows * ALZ_NB * 4));
+    CK(m.dev(&t->lat_sum, rows * 8));
+    CK(m.dev(&t->err5xx, rows * 8));
+    CK(m.dev(&t->count, rows * 8));
+    CK(m.dev(&t->hist, rows * ALZ_NB * 4));
     CK(cudaMemsetAsync(t->count, 0, rows * 8, h->stream));
     CK(cudaMemsetAsync(t->lat_sum, 0, rows * 8, h->stream));
     CK(cudaMemsetAsync(t->err5xx, 0, rows * 8, h->stream));
     CK(cudaMemsetAsync(t->hist, 0, rows * ALZ_NB * 4, h->stream));
   } else {
-    CK(cudaMalloc(&t->sect, rows * kSectPerRow * 32));
+    CK(m.dev(&t->sect, rows * kSectPerRow * 32));
     CK(cudaMemsetAsync(t->sect, 0, rows * kSectPerRow * 32, h->stream));
     // reversed rows are a few per cent of the traffic: a quarter-size dictionary is ample, and both
     // dictionaries draw rows from the one pool
     const uint32_t rev_cap = std::max<uint32_t>(1024u, dict_cap >> 2);
     t->dict_rev_mask = rev_cap - 1;
-    CK(cudaMalloc(&t->dict_rev, (size_t)rev_cap * sizeof(DictEnt)));
+    CK(m.dev(&t->dict_rev, (size_t)rev_cap * sizeof(DictEnt)));
     CK(cudaMemsetAsync(t->dict_rev, 0xFF, (size_t)rev_cap * sizeof(DictEnt), h->stream));
     const uint32_t host_cap = std::max<uint32_t>(1024u, dict_cap >> 3);   // host-keyed outbound pairs: rarer still
     t->dict_host_mask = host_cap - 1;
-    CK(cudaMalloc(&t->dict_host, (size_t)host_cap * sizeof(DictEnt)));
+    CK(m.dev(&t->dict_host, (size_t)host_cap * sizeof(DictEnt)));
     CK(cudaMemsetAsync(t->dict_host, 0xFF, (size_t)host_cap * sizeof(DictEnt), h->stream));
-    CK(cudaMalloc(&t->row_kind, rows));
+    CK(m.dev(&t->row_kind, rows));
     CK(cudaMemsetAsync(t->row_kind, 0, rows, h->stream));
     CK(cudaMemsetAsync(t->row_kind + max_rows + kPairRev, (int)kPairRev, 1, h->stream));   // sentinel rows of the free-marker key
     CK(cudaMemsetAsync(t->row_kind + max_rows + kPairHost, (int)kPairHost, 1, h->stream));
-    CK(cudaMalloc(&t->row_cnt, rows * 4)); CK(cudaMemsetAsync(t->row_cnt, 0, rows * 4, h->stream));
-    CK(cudaMalloc(&t->row_base, rows)); CK(cudaMemsetAsync(t->row_base, 0, rows, h->stream));
-    CK(cudaMalloc(&t->row_aux, rows * 4));
+    CK(m.dev(&t->row_cnt, rows * 4)); CK(cudaMemsetAsync(t->row_cnt, 0, rows * 4, h->stream));
+    CK(m.dev(&t->row_base, rows)); CK(cudaMemsetAsync(t->row_base, 0, rows, h->stream));
+    CK(m.dev(&t->row_aux, rows * 4));
   }
   CK(cudaMemsetAsync(t->dict, 0xFF, (size_t)dict_cap * sizeof(DictEnt), h->stream));
   return ALZ_OK;
-}
-static void free_table(AccTable* t) {
-  cudaFree(t->dict); cudaFree(t->dict_rev); cudaFree(t->dict_host); cudaFree(t->row_key); cudaFree(t->row_kind); cudaFree(t->lat_sum);
-  cudaFree(t->err5xx); cudaFree(t->count); cudaFree(t->row_cnt); cudaFree(t->row_base); cudaFree(t->row_aux); cudaFree(t->hist); cudaFree(t->sect);
-  memset(t, 0, sizeof(*t));
 }
 // all keys out of the dictionaries, row allocator back to zero (rows were zeroed by fold / gather)
 static int clear_dict(alz_handle* h, AccTable* t) {
@@ -124,7 +117,14 @@ extern "C" const char* alz_strerror(int s) {
   }
 }
 
-extern "C" const char* alz_last_cuda_error(alz_handle* h) { return h ? h->last_err.c_str() : ""; }
+// a copy taken under the lock: another thread may record a new error while the caller reads this one
+extern "C" const char* alz_last_cuda_error(alz_handle* h) {
+  if (!h) return "";
+  thread_local std::string copy;
+  std::lock_guard<std::mutex> g(h->err_mu);
+  copy = h->last_err;
+  return copy.c_str();
+}
 
 extern "C" int alz_create(const alz_config* cfg, alz_handle** out) {
   if (!cfg || !out || cfg->abi_version != ALZ_ABI_VERSION) return ALZ_E_INVAL;
@@ -152,87 +152,58 @@ extern "C" int alz_create(const alz_config* cfg, alz_handle** out) {
   cudaDeviceProp prop;
   CKC(cudaGetDeviceProperties(&prop, h->device));
   h->sms = prop.multiProcessorCount;
-  CKC(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
-  CKC(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
+  Owned& m = h->mem;
+  CKC(m.stream(&h->own_stream));
+  CKC(m.stream(&h->copy_stream));
   h->stream = h->own_stream;
-  for (int b = 0; b < kStageSlots; ++b) {
-    CKC(cudaEventCreateWithFlags(&h->stage[b].copied, cudaEventDisableTiming));
-    CKC(cudaEventCreateWithFlags(&h->stage[b].consumed, cudaEventDisableTiming));
+  for (int b = 0; b < kStageSlots + kRawSlots; ++b) {
+    StageSlot& s = b < kStageSlots ? h->stage[b] : h->raw[b - kStageSlots];
+    CKC(m.event(&s.copied, cudaEventDisableTiming));
+    CKC(m.event(&s.consumed, cudaEventDisableTiming));
   }
-  for (int b = 0; b < kRawSlots; ++b) {
-    CKC(cudaEventCreateWithFlags(&h->raw[b].copied, cudaEventDisableTiming));
-    CKC(cudaEventCreateWithFlags(&h->raw[b].consumed, cudaEventDisableTiming));
-  }
-  CKC(cudaEventCreateWithFlags(&h->ev_tmp, cudaEventDisableTiming));
-  CKC(cudaEventCreateWithFlags(&h->ev_count, cudaEventDisableTiming));
-  CKC(cudaEventCreateWithFlags(&h->ev_patch, cudaEventDisableTiming));
-  for (int i = 0; i < 3; ++i) CKC(cudaEventCreate(&h->ev_t[i]));
+  CKC(m.event(&h->ev_count, cudaEventDisableTiming));
+  CKC(m.event(&h->ev_patch, cudaEventDisableTiming));
+  for (int i = 0; i < 3; ++i) CKC(m.event(&h->ev_t[i], cudaEventDefault));
 
   h->ep_cap = next_pow2(2ull * h->cfg.max_endpoints);
   h->ep_tab.assign(h->ep_cap, EpEntry{0u, 0u, 0u, 0u});
   h->ep_touched.assign(h->ep_cap, 0);
-  CKC(cudaMalloc(&h->d_ep, (size_t)h->ep_cap * sizeof(EpEntry)));
+  CKC(m.dev(&h->d_ep, (size_t)h->ep_cap * sizeof(EpEntry)));
   CKC(cudaMemsetAsync(h->d_ep, 0, (size_t)h->ep_cap * sizeof(EpEntry), h->stream));
   h->bloom_cnt.assign(ALZ_BLOOM_WORDS * 32u, 0);
-  CKC(cudaMalloc(&h->d_bloom, ALZ_BLOOM_WORDS * 4u));
+  CKC(m.dev(&h->d_bloom, ALZ_BLOOM_WORDS * 4u));
   CKC(cudaMemsetAsync(h->d_bloom, 0, ALZ_BLOOM_WORDS * 4u, h->stream));   // no pods yet: every source is unresolvable
-  CKC(cudaMallocHost(&h->h_bloom, ALZ_BLOOM_WORDS * 4u));
-  CKC(cudaMalloc(&h->d_ctr, sizeof(Counters)));
+  CKC(m.pinned(&h->h_bloom, ALZ_BLOOM_WORDS * 4u));
+  CKC(m.dev(&h->d_ctr, sizeof(Counters)));
   CKC(cudaMemsetAsync(h->d_ctr, 0, sizeof(Counters), h->stream));
-  CKC(cudaMalloc(&h->d_hot, sizeof(HotState)));
+  CKC(m.dev(&h->d_hot, sizeof(HotState)));
   CKC(cudaMemsetAsync(h->d_hot, 0, sizeof(HotState), h->stream));
   int rc;
   if (!(h->cfg.flags & ALZ_CFG_EAGER_JOIN)) {
     if ((rc = alloc_table(h, &h->pairs, h->cfg.max_pairs, &h->d_ctr->pair_rows, true)) != ALZ_OK) return fail(rc);
   }
   if ((rc = alloc_table(h, &h->edges, h->cfg.max_edges, &h->d_ctr->edge_rows, false)) != ALZ_OK) return fail(rc);
-  CKC(cudaMallocHost(&h->h_ctr, sizeof(Counters)));
+  CKC(m.pinned(&h->h_ctr, sizeof(Counters)));
   memset(h->h_ctr, 0, sizeof(Counters));
   for (int b = 0; b < 2; ++b) {
-    CKC(cudaMalloc(&h->d_keys[b], (size_t)h->cfg.max_edges * 8));
-    CKC(cudaMalloc(&h->d_rows[b], (size_t)h->cfg.max_edges * 4));
+    CKC(m.dev(&h->d_keys[b], (size_t)h->cfg.max_edges * 8));
+    CKC(m.dev(&h->d_rows[b], (size_t)h->cfg.max_edges * 4));
   }
   h->sort_tmp_bytes = sort_pairs_temp_bytes(h->cfg.max_edges);
-  CKC(cudaMalloc(&h->d_sort_tmp, h->sort_tmp_bytes));
-  CKC(cudaMalloc(&h->d_out, (size_t)h->cfg.max_edges * sizeof(alz_edge_out)));
+  CKC(m.dev(&h->d_sort_tmp, h->sort_tmp_bytes));
+  CKC(m.dev(&h->d_out, (size_t)h->cfg.max_edges * sizeof(alz_edge_out)));
   CKC(cudaStreamSynchronize(h->stream));
 #undef CKC
   *out = h;
   return ALZ_OK;
 }
 
-static void free_slot(StageSlot& s) {
-  cudaFree(s.d); cudaFree(s.d_aux);
-  if (s.h) cudaFreeHost(s.h);
-  if (s.copied) cudaEventDestroy(s.copied);
-  if (s.consumed) cudaEventDestroy(s.consumed);
-  s.h = s.d = s.d_aux = nullptr;
-  s.copied = s.consumed = nullptr;
-}
-
 extern "C" int alz_destroy(alz_handle* h) {
   if (!h) return ALZ_E_INVAL;
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();
-  alz_internal_free_comm(h);
-  alz_internal_free_gnn(h);
-  alz_internal_free_sock(h);
-  free_table(&h->pairs); free_table(&h->edges);
-  cudaFree(h->d_ep); cudaFree(h->d_ctr); cudaFree(h->d_hot); cudaFree(h->d_patch);
-  cudaFree(h->d_win); cudaFree(h->d_defer[0]); cudaFree(h->d_defer[1]); cudaFree(h->d_bloom);
-  if (h->h_bloom) cudaFreeHost(h->h_bloom);
-  if (h->h_patch) cudaFreeHost(h->h_patch);
-  if (h->h_ctr) cudaFreeHost(h->h_ctr);
-  for (int b = 0; b < 2; ++b) { cudaFree(h->d_keys[b]); cudaFree(h->d_rows[b]); }
-  for (int b = 0; b < kStageSlots; ++b) free_slot(h->stage[b]);
-  for (int b = 0; b < kRawSlots; ++b) free_slot(h->raw[b]);
-  if (h->ev_tmp) cudaEventDestroy(h->ev_tmp);
-  if (h->ev_count) cudaEventDestroy(h->ev_count);
-  if (h->ev_patch) cudaEventDestroy(h->ev_patch);
-  for (int i = 0; i < 3; ++i) if (h->ev_t[i]) cudaEventDestroy(h->ev_t[i]);
-  cudaFree(h->d_sort_tmp); cudaFree(h->d_out);
-  if (h->own_stream) cudaStreamDestroy(h->own_stream);
-  if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
+  // owners go in reverse declaration order (alz_handle.h): the optional states (the NCCL communicator before
+  // the comm buffers), the grown buffers and the staging slots, then h->mem, whose streams are released last
   delete h;
   return ALZ_OK;
 }
@@ -307,17 +278,21 @@ static void with_gpu_local_cpus(int device, F f) {
   if (bound) sched_setaffinity(0, sizeof(old), &old);
 }
 
-// pinned memory on the NUMA node of the handle's GPU
+// pinned memory on the NUMA node of `device`: allocated and first touched from the CPUs next to it
+static cudaError_t pinned_alloc_local(int device, size_t bytes, void** out) {
+  cudaError_t e = cudaSuccess;
+  with_gpu_local_cpus(device, [&] {
+    cudaSetDevice(device);
+    e = cudaMallocHost(out, bytes);
+    if (e == cudaSuccess) for (size_t o = 0; o < bytes; o += 4096) ((volatile char*)*out)[o] = 0;
+  });
+  return e;
+}
+
 extern "C" int alz_pinned_alloc_local(alz_handle* h, size_t bytes, void** out) {
   if (!h || !out || bytes == 0) return ALZ_E_INVAL;
   void* p = nullptr;
-  cudaError_t e = cudaSuccess;
-  with_gpu_local_cpus(h->device, [&] {
-    cudaSetDevice(h->device);
-    e = cudaMallocHost(&p, bytes);
-    if (e == cudaSuccess) for (size_t o = 0; o < bytes; o += 4096) ((volatile char*)p)[o] = 0;
-  });
-  if (e != cudaSuccess) return ALZ_E_NOMEM;
+  if (pinned_alloc_local(h->device, bytes, &p) != cudaSuccess) return ALZ_E_NOMEM;
   std::lock_guard<std::mutex> g(g_pin_mu);
   g_pinned.emplace_back((const char*)p, bytes);
   *out = p;
@@ -409,9 +384,6 @@ static void ep_mirror_del(alz_handle* h, uint32_t ip) {
   ep_touch(h, i);
 }
 
-struct EpPatch { uint32_t slot, pad[3]; EpEntry e; };
-static_assert(sizeof(EpPatch) == 32, "EpPatch layout");
-
 static int fold_locked(alz_handle* h);
 
 extern "C" int alz_table_commit(alz_handle* h) {
@@ -443,17 +415,10 @@ extern "C" int alz_table_commit(alz_handle* h) {
   // may hold millions)
   const size_t n = h->ep_touched_list.size();
   if (n == 0) return ALZ_OK;
-  if (n > h->patch_cap) {
-    CK(cudaEventSynchronize(h->ev_patch));
-    if (h->h_patch) cudaFreeHost(h->h_patch);
-    cudaFree(h->d_patch);
-    h->h_patch = h->d_patch = nullptr;
-    h->patch_cap = std::max<size_t>(1024, n * 2);
-    CK(cudaMallocHost(&h->h_patch, h->patch_cap * sizeof(EpPatch)));
-    CK(cudaMalloc(&h->d_patch, h->patch_cap * sizeof(EpPatch)));
-  }
+  CK(h->h_patch.ensure(n, h->stream, std::max<size_t>(1024, n * 2)));
+  CK(h->d_patch.ensure(n, h->stream, std::max<size_t>(1024, n * 2)));
   CK(cudaEventSynchronize(h->ev_patch));   // the previous commit's upload has left the pinned buffer
-  EpPatch* p = (EpPatch*)h->h_patch;
+  EpPatch* p = h->h_patch.get();
   for (size_t i = 0; i < n; ++i) {
     const uint32_t slot = h->ep_touched_list[i];
     p[i].slot = slot; p[i].pad[0] = p[i].pad[1] = p[i].pad[2] = 0;
@@ -461,9 +426,9 @@ extern "C" int alz_table_commit(alz_handle* h) {
     h->ep_touched[slot] = 0;
   }
   h->ep_touched_list.clear();
-  CK(cudaMemcpyAsync(h->d_patch, h->h_patch, n * sizeof(EpPatch), cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(h->d_patch.get(), p, n * sizeof(EpPatch), cudaMemcpyHostToDevice, h->stream));
   CK(cudaEventRecord(h->ev_patch, h->stream));
-  launch_ep_patch(h->d_ep, h->d_patch, (uint32_t)n, h->sms, h->stream);
+  launch_ep_patch(h->d_ep, h->d_patch.get(), (uint32_t)n, h->sms, h->stream);
   h->launches += 1;
   CK(cudaGetLastError());
   return ALZ_OK;
@@ -543,49 +508,61 @@ extern "C" int alz_submit_l7_packed_device(alz_handle* h, const alz_l7_rec16* d,
   return ingest_device(h, d, n, true, d_ovf);
 }
 
-// staging slot s ready for `bytes` (allocated on first use, pinned memory next to the GPU)
+// staging slot s ready for `bytes` (allocated on first use, pinned memory next to the GPU); published only
+// once every buffer exists
 static int ensure_slot(alz_handle* h, StageSlot& s, size_t bytes, size_t aux_bytes) {
   if (s.h) return ALZ_OK;
-  cudaError_t e = cudaSuccess;
-  with_gpu_local_cpus(h->device, [&] {
-    cudaSetDevice(h->device);
-    e = cudaMallocHost(&s.h, bytes);
-    if (e == cudaSuccess) for (size_t o = 0; o < bytes; o += 4096) ((volatile char*)s.h)[o] = 0;
-  });
-  if (e != cudaSuccess) { s.h = nullptr; h->last_err = cudaGetErrorString(e); return ALZ_E_NOMEM; }
-  CK(cudaMalloc(&s.d, bytes));
-  if (aux_bytes) CK(cudaMalloc(&s.d_aux, aux_bytes));
+  void* p = nullptr;
+  const cudaError_t e = pinned_alloc_local(h->device, bytes, &p);
+  if (e != cudaSuccess) return alz_error(h, ALZ_E_NOMEM, nullptr, cudaGetErrorString(e));
+  Owner hb(p, ResFree{Res::kPinned}), d, aux;
+  CK(alz_alloc(d, Res::kDev, bytes));
+  if (aux_bytes) CK(alz_alloc(aux, Res::kDev, aux_bytes));
+  s.d = std::move(d);
+  s.d_aux = std::move(aux);
+  s.h = std::move(hb);
   return ALZ_OK;
 }
 
-// Host records -> device -> ingest, in chunks of max_batch, through the staging slots. rec_bytes = 32
-// (alz_l7_rec) or 16 (alz_l7_rec16).
-static int submit_host(alz_handle* h, const void* recs, size_t n, size_t rec_bytes, const uint64_t* d_ovf) {
+// Host records -> device -> ingest, in chunks through the staging slots. rec_bytes = 32 (alz_l7_rec) or
+// 16 (alz_l7_rec16); raw: ALZ_BPF_L7_EVENT_SIZE-byte samples through the raw slots, compacted into 32-B
+// records on the device before the ingest. A chunk is as many records as fit the byte size of max_batch
+// 32-B records.
+static int submit_staged(alz_handle* h, const void* recs, size_t n, size_t rec_bytes, bool raw, const uint64_t* d_ovf) {
+  StageSlot* slots = raw ? h->raw : h->stage;
+  const int n_slots = raw ? kRawSlots : kStageSlots;
+  uint64_t& next_turn = raw ? h->raw_turn : h->stage_turn;
   const bool direct = is_lib_pinned(recs, n * rec_bytes);
-  const size_t slot_bytes = (size_t)h->cfg.max_batch * sizeof(alz_l7_rec);
-  const size_t per = slot_bytes / rec_bytes;   // records per chunk (a 16-B chunk holds twice as many)
+  const size_t per = std::max<size_t>(1, (size_t)h->cfg.max_batch * sizeof(alz_l7_rec) / rec_bytes);
   size_t done = 0;
   while (done < n) {
     const size_t m = std::min(per, n - done);
     uint64_t turn;
-    { std::lock_guard<std::mutex> t(h->turn_mu); turn = h->stage_turn++; }
-    StageSlot& s = h->stage[turn % kStageSlots];
+    { std::lock_guard<std::mutex> t(h->turn_mu); turn = next_turn++; }
+    StageSlot& s = slots[turn % n_slots];
     std::lock_guard<std::mutex> own(s.mu);
-    int rc = ensure_slot(h, s, slot_bytes, 0);
+    int rc = ensure_slot(h, s, per * rec_bytes, raw ? per * sizeof(alz_l7_rec) : 0);
     if (rc != ALZ_OK) return rc;
     const void* src = (const char*)recs + done * rec_bytes;
     if (!direct) {
       CK(cudaEventSynchronize(s.copied));      // the previous H2D out of this pinned buffer is done
-      memcpy(s.h, src, m * rec_bytes);         // in parallel with other submitting threads
-      src = s.h;
+      memcpy(s.h.get(), src, m * rec_bytes);   // in parallel with other submitting threads
+      src = s.h.get();
     }
     {
       std::lock_guard<std::mutex> g(h->mu);
+      // the copy of chunk k+1 overlaps the (compaction +) ingest of chunk k (two slots or more, two streams)
       CK(cudaStreamWaitEvent(h->copy_stream, s.consumed, 0));   // the kernel that read s.d
-      CK(cudaMemcpyAsync(s.d, src, m * rec_bytes, cudaMemcpyHostToDevice, h->copy_stream));
+      CK(cudaMemcpyAsync(s.d.get(), src, m * rec_bytes, cudaMemcpyHostToDevice, h->copy_stream));
       CK(cudaEventRecord(s.copied, h->copy_stream));
       CK(cudaStreamWaitEvent(h->stream, s.copied, 0));
-      rc = ingest_device(h, s.d, m, rec_bytes == sizeof(alz_l7_rec16), d_ovf);
+      const void* d = s.d.get();
+      if (raw) {
+        launch_compact_raw((const uint8_t*)d, m, (alz_l7_rec*)s.d_aux.get(), h->sms, h->stream);
+        h->launches += 1;
+        d = s.d_aux.get();
+      }
+      rc = ingest_device(h, d, m, rec_bytes == sizeof(alz_l7_rec16), d_ovf);
       if (rc != ALZ_OK) return rc;
       CK(cudaEventRecord(s.consumed, h->stream));
     }
@@ -598,7 +575,7 @@ static int submit_host(alz_handle* h, const void* recs, size_t n, size_t rec_byt
 extern "C" int alz_submit_l7(alz_handle* h, const alz_l7_rec* recs, size_t n) {
   if (!h || (!recs && n)) return ALZ_E_INVAL;
   CK(cudaSetDevice(h->device));
-  return submit_host(h, recs, n, sizeof(alz_l7_rec), nullptr);
+  return submit_staged(h, recs, n, sizeof(alz_l7_rec), false, nullptr);
 }
 
 extern "C" int alz_submit_l7_packed(alz_handle* h, const alz_l7_rec16* recs, size_t n, const uint64_t* ovf, size_t n_ovf) {
@@ -611,7 +588,7 @@ extern "C" int alz_submit_l7_packed(alz_handle* h, const alz_l7_rec16* recs, siz
     CK(cudaMemcpyAsync(d_ovf, ovf, n_ovf * 8, cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));   // ovf is caller memory (possibly pageable): done with it before returning
   }
-  int rc = submit_host(h, recs, n, sizeof(alz_l7_rec16), d_ovf);
+  int rc = submit_staged(h, recs, n, sizeof(alz_l7_rec16), false, d_ovf);
   if (d_ovf) { std::lock_guard<std::mutex> g(h->mu); cudaFreeAsync(d_ovf, h->stream); }
   return rc;
 }
@@ -641,42 +618,7 @@ extern "C" long alz_pack_l7(const alz_l7_rec* recs, size_t n, alz_l7_rec16* out,
 extern "C" int alz_submit_l7_raw(alz_handle* h, const void* raw, size_t n) {
   if (!h || (!raw && n)) return ALZ_E_INVAL;
   CK(cudaSetDevice(h->device));
-  // raw chunk: as many samples as fit the byte size of one compact staging buffer
-  const size_t chunk = std::max<size_t>(1, ((size_t)h->cfg.max_batch * sizeof(alz_l7_rec)) / ALZ_BPF_L7_EVENT_SIZE);
-  const bool direct = is_lib_pinned(raw, n * ALZ_BPF_L7_EVENT_SIZE);
-  const uint8_t* p = (const uint8_t*)raw;
-  size_t done = 0;
-  while (done < n) {
-    const size_t m = std::min(chunk, n - done);
-    uint64_t turn;
-    { std::lock_guard<std::mutex> t(h->turn_mu); turn = h->raw_turn++; }
-    StageSlot& s = h->raw[turn % kRawSlots];
-    std::lock_guard<std::mutex> own(s.mu);
-    int rc = ensure_slot(h, s, chunk * ALZ_BPF_L7_EVENT_SIZE, chunk * sizeof(alz_l7_rec));
-    if (rc != ALZ_OK) return rc;
-    const void* src = p + done * ALZ_BPF_L7_EVENT_SIZE;
-    if (!direct) {
-      CK(cudaEventSynchronize(s.copied));
-      memcpy(s.h, src, m * ALZ_BPF_L7_EVENT_SIZE);
-      src = s.h;
-    }
-    {
-      std::lock_guard<std::mutex> g(h->mu);
-      // the copy of chunk k+1 overlaps the compaction + ingest of chunk k (two slots, two streams)
-      CK(cudaStreamWaitEvent(h->copy_stream, s.consumed, 0));
-      CK(cudaMemcpyAsync(s.d, src, m * ALZ_BPF_L7_EVENT_SIZE, cudaMemcpyHostToDevice, h->copy_stream));
-      CK(cudaEventRecord(s.copied, h->copy_stream));
-      CK(cudaStreamWaitEvent(h->stream, s.copied, 0));
-      launch_compact_raw((const uint8_t*)s.d, m, (alz_l7_rec*)s.d_aux, h->sms, h->stream);
-      h->launches += 1;
-      rc = ingest_device(h, s.d_aux, m, false, nullptr);
-      if (rc != ALZ_OK) return rc;
-      CK(cudaEventRecord(s.consumed, h->stream));
-    }
-    done += m;
-  }
-  if (direct) CK(cudaStreamSynchronize(h->copy_stream));
-  return ALZ_OK;
+  return submit_staged(h, raw, n, ALZ_BPF_L7_EVENT_SIZE, true, nullptr);
 }
 
 // ---- window result ---------------------------------------------------------------------------
@@ -727,7 +669,6 @@ static int window_roll(alz_handle* h) {
   h->launches += 1;
   const uint32_t n_def = std::min<uint32_t>(h->h_ctr->defer_count, h->defer_cap);   // read with the edge count
   CK(cudaMemsetAsync(&h->d_ctr->defer_count, 0, 4, h->stream));
-  h->deferred_last = 0;
   if (n_def == 0) return ALZ_OK;
   const alz_l7_rec* src = h->d_defer[h->defer_cur];
   h->defer_cur ^= 1;
@@ -844,16 +785,14 @@ extern "C" int alz_window_clock(alz_handle* h, uint64_t first_kernel_ns, uint64_
   CK(cudaSetDevice(h->device));
   if (h->pending_since_fold != 0 || h->h_ctr->defer_count != 0) return ALZ_E_STATE;   // only between windows
   if (window_ns == 0) { h->win_on = false; return ALZ_OK; }
-  if (!h->d_win) {
-    CK(cudaMalloc(&h->d_win, 3 * sizeof(uint64_t)));
-    h->defer_cap = 2u * h->cfg.max_batch;
-    for (int b = 0; b < 2; ++b) CK(cudaMalloc(&h->d_defer[b], (size_t)h->defer_cap * sizeof(alz_l7_rec)));
-  }
+  h->defer_cap = 2u * h->cfg.max_batch;
+  for (int b = 0; b < 2; ++b)   // each allocated once; a retry after a failure allocates only what is missing
+    if (!h->d_defer[b]) CK(h->mem.dev(&h->d_defer[b], (size_t)h->defer_cap * sizeof(alz_l7_rec)));
+  if (!h->d_win) CK(h->mem.dev(&h->d_win, 3 * sizeof(uint64_t)));
   const uint64_t init[3] = {0ull, window_ns, 0ull};
   CK(cudaMemcpyAsync(h->d_win, init, sizeof(init), cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   h->win_off = first_user_ns - first_kernel_ns;
-  h->win_len = window_ns;
   h->win_on = true;
   return ALZ_OK;
 }
@@ -884,8 +823,8 @@ extern "C" uint32_t alz_owner_rank(uint32_t saddr, uint32_t nranks) { return own
 extern "C" int alz_dev_alloc(alz_handle* h, size_t bytes, void** out) {
   if (!h || !out) return ALZ_E_INVAL;
   CK(cudaSetDevice(h->device));
-  cudaError_t e = cudaMalloc(out, bytes);
-  if (e != cudaSuccess) { h->last_err = cudaGetErrorString(e); return ALZ_E_NOMEM; }
+  const cudaError_t e = cudaMalloc(out, bytes);   // the caller's: freed with alz_dev_free
+  if (e != cudaSuccess) return alz_error(h, ALZ_E_NOMEM, nullptr, cudaGetErrorString(e));
   return ALZ_OK;
 }
 extern "C" int alz_dev_free(alz_handle* h, void* p) {
@@ -912,33 +851,33 @@ extern "C" int alz_memcpy_d2h(alz_handle* h, void* dst, const void* src, size_t 
 }
 
 struct alz_synth_dev {
-  alz_synth_view view;  // device pointers
-  void* bufs[6];
+  alz_synth_view view;  // device pointers into mem
+  Owned mem;
 };
 
 extern "C" int alz_synth_dev_create(alz_handle* h, const alz_synth_topo* t, alz_synth_dev** out) {
   if (!h || !t || !out) return ALZ_E_INVAL;
   std::lock_guard<std::mutex> g(h->mu);
   CK(cudaSetDevice(h->device));
-  alz_synth_dev* d = new (std::nothrow) alz_synth_dev();
+  std::unique_ptr<alz_synth_dev> d(new (std::nothrow) alz_synth_dev());
   if (!d) return ALZ_E_NOMEM;
-  memset(d, 0, sizeof(*d));
   d->view = t->view;
   const size_t E = t->n_edges;
   const void* src[6] = {t->edge_saddr, t->edge_daddr, t->edge_flags, t->alias_thresh, t->alias_idx, t->lat_q};
   const size_t bytes[6] = {E * 4, E * 4, E, E * 4, E * 4, (ALZ_SYNTH_LATQ + 1) * 8};
+  void* bufs[6];
   for (int i = 0; i < 6; ++i) {
-    CK(cudaMalloc(&d->bufs[i], bytes[i]));
-    CK(cudaMemcpyAsync(d->bufs[i], src[i], bytes[i], cudaMemcpyHostToDevice, h->stream));
+    CK(d->mem.dev(&bufs[i], bytes[i]));
+    CK(cudaMemcpyAsync(bufs[i], src[i], bytes[i], cudaMemcpyHostToDevice, h->stream));
   }
   CK(cudaStreamSynchronize(h->stream));   // the sources are pageable caller memory
-  d->view.edge_saddr = (const uint32_t*)d->bufs[0];
-  d->view.edge_daddr = (const uint32_t*)d->bufs[1];
-  d->view.edge_flags = (const uint8_t*)d->bufs[2];
-  d->view.alias_thresh = (const uint32_t*)d->bufs[3];
-  d->view.alias_idx = (const uint32_t*)d->bufs[4];
-  d->view.lat_q = (const uint64_t*)d->bufs[5];
-  *out = d;
+  d->view.edge_saddr = (const uint32_t*)bufs[0];
+  d->view.edge_daddr = (const uint32_t*)bufs[1];
+  d->view.edge_flags = (const uint8_t*)bufs[2];
+  d->view.alias_thresh = (const uint32_t*)bufs[3];
+  d->view.alias_idx = (const uint32_t*)bufs[4];
+  d->view.lat_q = (const uint64_t*)bufs[5];
+  *out = d.release();
   return ALZ_OK;
 }
 extern "C" int alz_synth_dev_fill(alz_handle* h, alz_synth_dev* d, uint64_t first, uint64_t n, alz_l7_rec* dev_out) {
@@ -956,8 +895,9 @@ extern "C" int alz_synth_dev_fill_owned(alz_handle* h, alz_synth_dev* d, uint64_
   if (!h || !d || !dev_out || !n_written || !n_scanned || nranks == 0 || rank >= nranks) return ALZ_E_INVAL;
   std::lock_guard<std::mutex> g(h->mu);
   CK(cudaSetDevice(h->device));
+  Owned scratch;   // freed on every return, with the device still current
   unsigned long long* d_cnt = nullptr;
-  CK(cudaMalloc(&d_cnt, 8));
+  CK(scratch.dev(&d_cnt, 8));
   CK(cudaMemsetAsync(d_cnt, 0, 8, h->stream));
   const uint64_t chunk = std::max<uint64_t>(1u << 20, want / 4);
   unsigned long long got = 0;
@@ -968,7 +908,6 @@ extern "C" int alz_synth_dev_fill_owned(alz_handle* h, alz_synth_dev* d, uint64_
     CK(cudaMemcpyAsync(&got, d_cnt, 8, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
   }
-  cudaFree(d_cnt);
   *n_written = got < want ? got : want;
   *n_scanned = scanned;
   return ALZ_OK;
@@ -976,7 +915,6 @@ extern "C" int alz_synth_dev_fill_owned(alz_handle* h, alz_synth_dev* d, uint64_
 extern "C" int alz_synth_dev_destroy(alz_handle* h, alz_synth_dev* d) {
   if (!h || !d) return ALZ_E_INVAL;
   cudaSetDevice(h->device);
-  for (int i = 0; i < 6; ++i) cudaFree(d->bufs[i]);
   delete d;
   return ALZ_OK;
 }

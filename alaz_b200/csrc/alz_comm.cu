@@ -285,6 +285,8 @@ __global__ void __launch_bounds__(256) consume_window_kernel(const MergeInfo* __
 }  // namespace
 
 struct alz_comm_state {
+  ~alz_comm_state() { if (comm && g_nccl.CommDestroy) g_nccl.CommDestroy(comm); }   // before the buffers below go
+  Owned mem;
   ncclComm_t comm = nullptr;
   uint32_t* d_counts = nullptr;   // [nranks]
   uint32_t* h_counts = nullptr;   // pinned
@@ -301,29 +303,18 @@ struct alz_comm_state {
   size_t gather_cap = 0;          // keys
   // default path
   alz_edge_out* d_send = nullptr; // [1 + block_rows_for(max_edges)]: header row + local sorted rows (+ head room)
-  alz_edge_out* d_recv = nullptr; // [R * (1 + cap_r)]
-  size_t recv_rows = 0;           // allocated rows of d_recv
+  GrowBuf<alz_edge_out> d_recv;   // [R * (1 + cap_r)]
   uint32_t cap_r = 0;             // rows per rank block of the next collective (0 = not known yet)
   BlockHeader* h_hdr = nullptr;   // pinned
   MergeInfo* d_info = nullptr;
   MergeInfo* h_info = nullptr;    // pinned
 };
+void StateDelete::operator()(alz_comm_state* c) const { delete c; }
 
-#define CK(expr)                                                                       \
-  do {                                                                                 \
-    cudaError_t _e = (expr);                                                           \
-    if (_e != cudaSuccess) {                                                           \
-      h->last_err = std::string(#expr) + ": " + cudaGetErrorString(_e);                \
-      return ALZ_E_CUDA;                                                               \
-    }                                                                                  \
-  } while (0)
 #define NK(expr)                                                                       \
   do {                                                                                 \
-    ncclResult_t _r = (expr);                                                          \
-    if (_r != ncclSuccess) {                                                           \
-      h->last_err = std::string(#expr) + ": " + g_nccl.GetErrorString(_r);             \
-      return ALZ_E_NCCL;                                                               \
-    }                                                                                  \
+    const ncclResult_t _r = (expr);                                                    \
+    if (_r != ncclSuccess) return alz_error(h, ALZ_E_NCCL, #expr, g_nccl.GetErrorString(_r)); \
   } while (0)
 
 extern "C" int alz_comm_unique_id(void* out_id) {
@@ -346,58 +337,47 @@ extern "C" int alz_comm_init(alz_handle* h, int nranks, int rank, const void* id
   if (!h || !id_bytes || nranks < 1 || rank < 0 || rank >= nranks) return ALZ_E_INVAL;
   std::lock_guard<std::mutex> g(h->mu);
   if (h->comm) return ALZ_E_STATE;
-  if (!load_nccl()) { h->last_err = "dlopen(libnccl.so.2) failed"; return ALZ_E_NCCL; }
+  if (!load_nccl()) return alz_error(h, ALZ_E_NCCL, nullptr, "dlopen(libnccl.so.2) failed");
   CK(cudaSetDevice(h->device));
-  alz_comm_state* c = new alz_comm_state();
+  // built here and published only when complete: a failure leaves the handle single-rank, and the caller may retry
+  StatePtr<alz_comm_state> c(new alz_comm_state());
   ncclUniqueId id;
   memcpy(&id, id_bytes, sizeof(id));
-  ncclResult_t r = g_nccl.CommInitRank(&c->comm, nranks, id, rank);
-  if (r != ncclSuccess) { h->last_err = g_nccl.GetErrorString(r); delete c; return ALZ_E_NCCL; }
-  h->comm = c;
-  h->comm_nranks = nranks;
-  h->comm_rank = rank;
+  ncclComm_t comm = nullptr;
+  NK(g_nccl.CommInitRank(&comm, nranks, id, rank));
+  c->comm = comm;
   const size_t me = h->cfg.max_edges;
   c->gather_cap = me;  // every rank holds the merged graph, so max_edges bounds the gathered keys too
-  CK(cudaMalloc(&c->d_counts, sizeof(uint32_t) * nranks));
-  CK(cudaMallocHost(&c->h_counts, sizeof(uint32_t) * nranks));
-  CK(cudaMalloc(&c->d_gather, me * 8 * 2));
+  Owned& m = c->mem;
+  CK(m.dev(&c->d_counts, sizeof(uint32_t) * nranks));
+  CK(m.pinned(&c->h_counts, sizeof(uint32_t) * nranks));
+  CK(m.dev(&c->d_gather, me * 8 * 2));
   c->d_sorted = c->d_gather + me;
-  CK(cudaMalloc(&c->d_flags, me * 4));
-  CK(cudaMalloc(&c->d_pos, me * 4));
-  CK(cudaMalloc(&c->d_can_keys, me * 8));
-  CK(cudaMalloc(&c->d_can, me * kCanWords * 8));
-  CK(cudaMalloc(&c->d_iota, me * 4));
-  CK(cudaMalloc(&c->d_vals, me * 4));
+  CK(m.dev(&c->d_flags, me * 4));
+  CK(m.dev(&c->d_pos, me * 4));
+  CK(m.dev(&c->d_can_keys, me * 8));
+  CK(m.dev(&c->d_can, me * kCanWords * 8));
+  CK(m.dev(&c->d_iota, me * 4));
+  CK(m.dev(&c->d_vals, me * 4));
   c->tmp_bytes = std::max(sort_pairs_temp_bytes((uint32_t)me), scan_temp_bytes((uint32_t)me));
-  CK(cudaMalloc(&c->d_tmp, c->tmp_bytes));
+  CK(m.dev(&c->d_tmp, c->tmp_bytes));
   // a block is sized from the largest rank's count plus head room: up to block_rows_for(max_edges) rows are SENT
   // from here even when this rank has fewer (max_edges must be the same on every rank)
   const size_t send_rows = (size_t)block_rows_for(me) + 1;
-  CK(cudaMalloc(&c->d_send, send_rows * sizeof(alz_edge_out)));
+  CK(m.dev(&c->d_send, send_rows * sizeof(alz_edge_out)));
   CK(cudaMemset(c->d_send, 0, send_rows * sizeof(alz_edge_out)));
-  CK(cudaMallocHost(&c->h_hdr, sizeof(alz_edge_out)));
-  CK(cudaMalloc(&c->d_info, sizeof(MergeInfo)));
-  CK(cudaMallocHost(&c->h_info, sizeof(MergeInfo)));
+  CK(m.pinned(&c->h_hdr, sizeof(alz_edge_out)));
+  CK(m.dev(&c->d_info, sizeof(MergeInfo)));
+  CK(m.pinned(&c->h_info, sizeof(MergeInfo)));
+  h->comm = std::move(c);
+  h->comm_nranks = nranks;
+  h->comm_rank = rank;
   return ALZ_OK;
-}
-
-void alz_internal_free_comm(alz_handle* h) {
-  alz_comm_state* c = h->comm;
-  if (!c) return;
-  if (c->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(c->comm);
-  cudaFree(c->d_counts); if (c->h_counts) cudaFreeHost(c->h_counts);
-  cudaFree(c->d_gather); cudaFree(c->d_flags); cudaFree(c->d_pos); cudaFree(c->d_can_keys);
-  cudaFree(c->d_can); cudaFree(c->d_iota); cudaFree(c->d_vals); cudaFree(c->d_tmp);
-  cudaFree(c->d_send); cudaFree(c->d_recv); cudaFree(c->d_info);
-  if (c->h_hdr) cudaFreeHost(c->h_hdr);
-  if (c->h_info) cudaFreeHost(c->h_info);
-  delete c;
-  h->comm = nullptr;
 }
 
 // General path: keys may live on several ranks. Local live edges are sorted in d_keys[1] / d_rows[1].
 static int merge_allreduce(alz_handle* h) {
-  alz_comm_state* c = h->comm;
+  alz_comm_state* c = h->comm.get();
   const int R = h->comm_nranks;
   cudaStream_t s = h->stream;
   const unsigned grid = (unsigned)h->sms * 4;
@@ -470,7 +450,7 @@ static int merge_allreduce(alz_handle* h) {
 // (rows), h->n_live of them; local_rc is this rank's status so far. Every rank enters the collective whatever
 // its own status, so nobody is left waiting in NCCL, and all ranks return the same failure.
 int alz_internal_merge_ranks(alz_handle* h, int local_rc) {
-  alz_comm_state* c = h->comm;
+  alz_comm_state* c = h->comm.get();
   if (!c || h->comm_nranks <= 1) return ALZ_E_UNSUPPORTED;
   const int R = h->comm_nranks;
   if (R > 64) return ALZ_E_UNSUPPORTED;
@@ -498,18 +478,12 @@ int alz_internal_merge_ranks(alz_handle* h, int local_rc) {
     c->h_hdr->magic = kHdrMagic; c->h_hdr->count = n_local; c->h_hdr->status = local_rc;
     CK(cudaMemcpyAsync(c->d_send, c->h_hdr, sizeof(alz_edge_out), cudaMemcpyHostToDevice, s));
     const size_t block_rows = (size_t)c->cap_r + 1;
-    if (block_rows * R > c->recv_rows) {
-      CK(cudaStreamSynchronize(s));
-      cudaFree(c->d_recv);
-      c->d_recv = nullptr;
-      c->recv_rows = block_rows * R;
-      CK(cudaMalloc(&c->d_recv, c->recv_rows * sizeof(alz_edge_out)));
-    }
+    CK(c->d_recv.ensure(block_rows * R, s));
     CK(cudaMemsetAsync(c->d_info, 0, sizeof(MergeInfo), s));
     // the single exchange step: every rank's header + its first cap_r rows
-    NK(g_nccl.AllGather(c->d_send, c->d_recv, block_rows * kRowWords64, ncclUint64, c->comm, s));
+    NK(g_nccl.AllGather(c->d_send, c->d_recv.get(), block_rows * kRowWords64, ncclUint64, c->comm, s));
     h->collective_bytes_last += (uint64_t)block_rows * R * kRowBytes;
-    merge_blocks_kernel<<<grid, 256, 0, s>>>(c->d_recv, c->cap_r, (uint32_t)R, h->d_out, h->cfg.max_edges, c->d_info);
+    merge_blocks_kernel<<<grid, 256, 0, s>>>(c->d_recv.get(), c->cap_r, (uint32_t)R, h->d_out, h->cfg.max_edges, c->d_info);
     consume_window_kernel<<<grid, 256, 0, s>>>(c->d_info, h->edges, h->d_rows[1], n_local);
     h->launches += 2;
     CK(cudaGetLastError());

@@ -520,6 +520,7 @@ __global__ void __launch_bounds__(256) edge_score_kernel(const alz_edge_out* __r
 }  // namespace
 
 struct alz_gnn_state {
+  Owned mem;
   uint32_t cap_e = 0, cap_v = 0;
   uint64_t *d_nk = nullptr, *d_nk_sorted = nullptr, *d_nodes = nullptr, *d_dst_key = nullptr, *d_dst_sorted = nullptr;
   uint32_t *d_flags = nullptr, *d_pos = nullptr, *d_iota = nullptr, *d_vals = nullptr, *d_src_idx = nullptr;
@@ -536,46 +537,40 @@ struct alz_gnn_state {
   bool n_v_known = true;
   uint32_t* d_nv = nullptr;      // node count of the last pass, on the device
 };
+void StateDelete::operator()(alz_gnn_state* g) const { delete g; }
 
-#define CK(expr)                                                                       \
-  do {                                                                                 \
-    cudaError_t _e = (expr);                                                           \
-    if (_e != cudaSuccess) {                                                           \
-      h->last_err = std::string(#expr) + ": " + cudaGetErrorString(_e);                \
-      return ALZ_E_CUDA;                                                               \
-    }                                                                                  \
-  } while (0)
-
-static int gnn_init_impl(alz_handle* h) {
-  alz_gnn_state* g = new alz_gnn_state();
-  h->gnn = g;
+// built on first use and published only when complete: after a failed allocation the next call starts again
+static int gnn_init(alz_handle* h) {
+  if (h->gnn) return ALZ_OK;
+  StatePtr<alz_gnn_state> g(new alz_gnn_state());
+  Owned& m = g->mem;
   g->cap_e = h->cfg.max_edges;
   g->cap_v = 2 * h->cfg.max_edges;
   const size_t E = g->cap_e, V = g->cap_v;
-  CK(cudaMalloc(&g->d_nk, V * 8));
-  CK(cudaMalloc(&g->d_nk_sorted, V * 8));
-  CK(cudaMalloc(&g->d_nodes, V * 8));
-  CK(cudaMalloc(&g->d_dst_key, E * 8));
-  CK(cudaMalloc(&g->d_dst_sorted, E * 8));
-  CK(cudaMalloc(&g->d_flags, V * 4));
-  CK(cudaMalloc(&g->d_pos, V * 4));
-  CK(cudaMalloc(&g->d_iota, V * 4));
-  CK(cudaMalloc(&g->d_vals, V * 4));
-  CK(cudaMalloc(&g->d_src_idx, E * 4));
-  CK(cudaMalloc(&g->d_in_deg, (V + 1) * 4));
-  CK(cudaMalloc(&g->d_rowptr, (V + 1) * 4));
-  CK(cudaMalloc(&g->d_col, E * 4));
-  CK(cudaMalloc(&g->d_sorted_edge, E * 4));
-  CK(cudaMalloc(&g->d_stats, V * 8 * 8));
-  for (int i = 0; i < 3; ++i) CK(cudaMalloc(&g->d_h[i], V * D * 4));
-  CK(cudaMalloc(&g->d_scores, E * 4));
-  CK(cudaMalloc(&g->d_nv, 4));
+  CK(m.dev(&g->d_nk, V * 8));
+  CK(m.dev(&g->d_nk_sorted, V * 8));
+  CK(m.dev(&g->d_nodes, V * 8));
+  CK(m.dev(&g->d_dst_key, E * 8));
+  CK(m.dev(&g->d_dst_sorted, E * 8));
+  CK(m.dev(&g->d_flags, V * 4));
+  CK(m.dev(&g->d_pos, V * 4));
+  CK(m.dev(&g->d_iota, V * 4));
+  CK(m.dev(&g->d_vals, V * 4));
+  CK(m.dev(&g->d_src_idx, E * 4));
+  CK(m.dev(&g->d_in_deg, (V + 1) * 4));
+  CK(m.dev(&g->d_rowptr, (V + 1) * 4));
+  CK(m.dev(&g->d_col, E * 4));
+  CK(m.dev(&g->d_sorted_edge, E * 4));
+  CK(m.dev(&g->d_stats, V * 8 * 8));
+  for (int i = 0; i < 3; ++i) CK(m.dev(&g->d_h[i], V * D * 4));
+  CK(m.dev(&g->d_scores, E * 4));
+  CK(m.dev(&g->d_nv, 4));
   g->tmp_bytes = std::max(sort_pairs_temp_bytes((uint32_t)V), scan_temp_bytes((uint32_t)V + 1));
-  CK(cudaMalloc(&g->d_tmp, g->tmp_bytes));
+  CK(m.dev(&g->d_tmp, g->tmp_bytes));
   const Weights w = make_weights();
   for (int l = 0; l < 2; ++l) {
-    CK(cudaMalloc(&g->d_W[l], 128 * D * 4));
-    CK(cudaMalloc(&g->d_b[l], D * 4));
+    CK(m.dev(&g->d_W[l], 128 * D * 4));
+    CK(m.dev(&g->d_b[l], D * 4));
     CK(cudaMemcpyAsync(g->d_W[l], w.W[l].data(), 128 * D * 4, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(g->d_b[l], w.b[l].data(), D * 4, cudaMemcpyHostToDevice, h->stream));
   }
@@ -592,39 +587,18 @@ static int gnn_init_impl(alz_handle* h) {
           can[off] = hi;
           can[tc::TN * tc::TK + off] = lo;
         }
-      CK(cudaMalloc(&g->d_Wcan[l], 2 * tc::B_BYTES));
+      CK(m.dev(&g->d_Wcan[l], 2 * tc::B_BYTES));
       CK(cudaMemcpyAsync(g->d_Wcan[l], can.data(), 2 * tc::B_BYTES, cudaMemcpyHostToDevice, h->stream));
       CK(cudaStreamSynchronize(h->stream));   // `can` is rewritten for the next layer
     }
     CK(cudaFuncSetAttribute(tc::sage_layer_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::SMEM_TC));
   }
-  CK(cudaMalloc(&g->d_a, 132 * 4));
+  CK(m.dev(&g->d_a, 132 * 4));
   CK(cudaMemcpyAsync(g->d_a, w.a.data(), 132 * 4, cudaMemcpyHostToDevice, h->stream));
   CK(cudaStreamSynchronize(h->stream));     // the host-side weight vectors die with this frame
   g->c = w.c;
+  h->gnn = std::move(g);
   return ALZ_OK;
-}
-
-void alz_internal_free_gnn(alz_handle* h);
-// a half-built state never stays published: a failed allocation frees everything and the next call retries
-static int gnn_init(alz_handle* h) {
-  if (h->gnn) return ALZ_OK;
-  const int rc = gnn_init_impl(h);
-  if (rc != ALZ_OK) alz_internal_free_gnn(h);
-  return rc;
-}
-
-void alz_internal_free_gnn(alz_handle* h) {
-  alz_gnn_state* g = h->gnn;
-  if (!g) return;
-  cudaFree(g->d_nk); cudaFree(g->d_nk_sorted); cudaFree(g->d_nodes); cudaFree(g->d_dst_key); cudaFree(g->d_dst_sorted);
-  cudaFree(g->d_flags); cudaFree(g->d_pos); cudaFree(g->d_iota); cudaFree(g->d_vals); cudaFree(g->d_src_idx);
-  cudaFree(g->d_in_deg); cudaFree(g->d_rowptr); cudaFree(g->d_col); cudaFree(g->d_sorted_edge); cudaFree(g->d_stats);
-  for (int i = 0; i < 3; ++i) cudaFree(g->d_h[i]);
-  for (int l = 0; l < 2; ++l) { cudaFree(g->d_W[l]); cudaFree(g->d_b[l]); cudaFree(g->d_Wcan[l]); }
-  cudaFree(g->d_a); cudaFree(g->d_scores); cudaFree(g->d_tmp); cudaFree(g->d_nv);
-  delete g;
-  h->gnn = nullptr;
 }
 
 // CSR build + 2 layers + scoring over the last flushed window (h->d_out). Nothing here waits for the device:
@@ -635,7 +609,7 @@ static int bits_for(uint64_t x) { int b = 1; while (b < 64 && (x >> b) != 0) ++b
 static int gnn_run(alz_handle* h) {
   int rc = gnn_init(h);
   if (rc != ALZ_OK) return rc;
-  alz_gnn_state* g = h->gnn;
+  alz_gnn_state* g = h->gnn.get();
   cudaStream_t s = h->stream;
   const uint32_t n_e = h->last_n_edges;
   g->n_e = n_e;

@@ -1,6 +1,8 @@
 // alz_handle.h — the handle behind the C ABI: everything one GPU owns.
 #pragma once
+#include <algorithm>
 #include <cstdint>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <unordered_map>
@@ -11,22 +13,124 @@
 #include "../../include/alazgpu_synth.h"
 #include "alz_kernels.cuh"
 
+struct alz_handle;
+
+// ---- errors ------------------------------------------------------------------------------------------
+// Records "what: why" as the handle's last error and returns rc. The only writer of last_err: it takes
+// err_mu, because submitting threads may fail at the same time.
+int alz_error(alz_handle* h, int rc, const char* what, const char* why);
+
+#define CK(expr)                                                                       \
+  do {                                                                                 \
+    const cudaError_t _e = (expr);                                                     \
+    if (_e != cudaSuccess) return alz_error(h, ALZ_E_CUDA, #expr, cudaGetErrorString(_e)); \
+  } while (0)
+
+// ---- ownership ---------------------------------------------------------------------------------------
+// What the library takes from CUDA is held by owners. The structs handed to kernels by value (AccTable,
+// HotState, Counters, alz_synth_view, ...) keep raw pointers; the memory behind them belongs to an owner
+// beside them. An owner is destroyed only while its handle's device is current: one process may drive
+// several GPUs from several threads.
+enum class Res { kDev, kPinned, kEvent, kStream };
+struct ResFree {
+  Res kind = Res::kDev;
+  void operator()(void* p) const {
+    switch (kind) {
+      case Res::kDev: cudaFree(p); break;
+      case Res::kPinned: cudaFreeHost(p); break;
+      case Res::kEvent: cudaEventDestroy(static_cast<cudaEvent_t>(p)); break;
+      case Res::kStream: cudaStreamDestroy(static_cast<cudaStream_t>(p)); break;
+    }
+  }
+};
+using Owner = std::unique_ptr<void, ResFree>;
+
+// cudaMalloc / cudaMallocHost into o; o is left untouched on failure
+inline cudaError_t alz_alloc(Owner& o, Res kind, size_t bytes) {
+  void* p = nullptr;
+  const cudaError_t e = kind == Res::kPinned ? cudaMallocHost(&p, bytes) : cudaMalloc(&p, bytes);
+  if (e == cudaSuccess) o = Owner(p, ResFree{kind});
+  return e;
+}
+
+// A buffer of T that grows on demand (device or pinned)
+template <class T>
+struct GrowBuf {
+  explicit GrowBuf(Res kind = Res::kDev) : p(nullptr, ResFree{kind}) {}
+  T* get() const { return static_cast<T*>(p.get()); }
+  // at least n elements; a growth allocates max(n, grow) of them. Work in flight on `stream` may still use the
+  // old buffer, so it waits for the stream before freeing it; cap changes only once the allocation succeeded.
+  cudaError_t ensure(size_t n, cudaStream_t stream, size_t grow = 0) {
+    if (n <= cap) return cudaSuccess;
+    if (p) {
+      const cudaError_t e = cudaStreamSynchronize(stream);
+      if (e != cudaSuccess) return e;
+      p.reset();
+      cap = 0;
+    }
+    const size_t want = std::max(n, grow);
+    const cudaError_t e = alz_alloc(p, p.get_deleter().kind, want * sizeof(T));
+    if (e == cudaSuccess) cap = want;
+    return e;
+  }
+  Owner p;
+  size_t cap = 0;   // elements
+};
+
+// Everything a state allocated once, for its whole life. Released in reverse order of allocation, so a
+// handle's streams (created first) outlive its buffers and events.
+struct Owned {
+  ~Owned() { while (!items.empty()) items.pop_back(); }
+  template <class T> cudaError_t dev(T** out, size_t bytes) { return add(Res::kDev, reinterpret_cast<void**>(out), bytes); }
+  template <class T> cudaError_t pinned(T** out, size_t bytes) { return add(Res::kPinned, reinterpret_cast<void**>(out), bytes); }
+  cudaError_t event(cudaEvent_t* out, unsigned flags) {
+    cudaEvent_t e = nullptr;
+    const cudaError_t r = cudaEventCreateWithFlags(&e, flags);
+    if (r == cudaSuccess) { items.emplace_back(e, ResFree{Res::kEvent}); *out = e; }
+    return r;
+  }
+  cudaError_t stream(cudaStream_t* out) {
+    cudaStream_t s = nullptr;
+    const cudaError_t r = cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
+    if (r == cudaSuccess) { items.emplace_back(s, ResFree{Res::kStream}); *out = s; }
+    return r;
+  }
+
+ private:
+  cudaError_t add(Res kind, void** out, size_t bytes) {
+    Owner o;
+    const cudaError_t e = alz_alloc(o, kind, bytes);
+    if (e == cudaSuccess) { *out = o.get(); items.push_back(std::move(o)); }
+    return e;
+  }
+  std::vector<Owner> items;
+};
+
 struct HostEp {
   uint32_t state = 0;  // kEpPod | kEpSvc
   uint32_t pod = 0, svc = 0;
 };
 
+struct EpPatch { uint32_t slot, pad[3]; alz::EpEntry e; };
+static_assert(sizeof(EpPatch) == 32, "EpPatch layout");
+
 struct alz_gnn_state;   // alz_gnn.cu
 struct alz_sock_state;  // alz_sock.cu
 struct alz_comm_state;  // alz_comm.cu
+struct StateDelete {    // each defined beside its state
+  void operator()(alz_comm_state* c) const;
+  void operator()(alz_gnn_state* g) const;
+  void operator()(alz_sock_state* s) const;
+};
+template <class T> using StatePtr = std::unique_ptr<T, StateDelete>;
 
 // One host->device staging slot: pinned host buffer + device buffer. A submitting thread owns the slot
-// (mu) from the copy into the pinned buffer until its H2D and kernel are enqueued.
+// (mu) from the copy into the pinned buffer until its H2D and kernel are enqueued. The buffers are
+// published together (h last), so a slot with h is whole.
 struct StageSlot {
   std::mutex mu;
-  void* h = nullptr;
-  void* d = nullptr;
-  void* d_aux = nullptr;                  // raw path: compacted 32-B records
+  Owner h, d;
+  Owner d_aux;                            // raw path: compacted 32-B records
   cudaEvent_t copied = nullptr;           // H2D out of h done -> h may be rewritten
   cudaEvent_t consumed = nullptr;         // kernel that read d (and d_aux) done -> d may be rewritten
 };
@@ -36,9 +140,13 @@ constexpr int kRawSlots = 2;
 struct alz_handle {
   alz_config cfg{};
   int device = 0, sms = 0;
+  // streams, events and the fixed buffers of alz_create / alz_window_clock. Declared before every other
+  // owner, so destroyed after them: the streams go last.
+  Owned mem;
   cudaStream_t own_stream = nullptr, stream = nullptr, copy_stream = nullptr;
-  cudaEvent_t ev_tmp = nullptr, ev_count = nullptr;
-  std::string last_err;
+  cudaEvent_t ev_count = nullptr;
+  std::mutex err_mu;
+  std::string last_err;                   // written only by alz_error
 
   // Serialises everything that enqueues on `stream` or touches the bookkeeping below. Submitting threads
   // take it only around their enqueue; flush / commit / stats hold it for the whole call.
@@ -47,7 +155,6 @@ struct alz_handle {
   uint64_t stage_turn = 0, raw_turn = 0;
   StageSlot stage[kStageSlots];
   StageSlot raw[kRawSlots];
-  size_t raw_chunk = 0;                   // samples per raw slot
 
   // join build side: host mirror of the ClusterInfo maps and of the device's open-addressed table;
   // a commit patches only the slots that changed (alz_table_commit)
@@ -62,9 +169,8 @@ struct alz_handle {
   bool bloom_dirty = false;
   uint32_t* d_bloom = nullptr;            // ALZ_BLOOM_WORDS words
   uint32_t* h_bloom = nullptr;            // pinned staging
-  void* h_patch = nullptr;                // pinned: (slot, entry) records of one commit
-  void* d_patch = nullptr;
-  size_t patch_cap = 0;
+  GrowBuf<EpPatch> h_patch{Res::kPinned}; // (slot, entry) records of one commit
+  GrowBuf<EpPatch> d_patch;
   cudaEvent_t ev_patch = nullptr;
 
   // accumulators
@@ -84,12 +190,11 @@ struct alz_handle {
 
   // time-cut windows (alz_window_clock)
   bool win_on = false;
-  uint64_t win_off = 0, win_len = 0;      // first_user - first_kernel (mod 2^64), window length
+  uint64_t win_off = 0;                   // first_user - first_kernel (mod 2^64)
   uint64_t* d_win = nullptr;              // device WinClock {lo, len, ready}
   alz_l7_rec* d_defer[2] = {nullptr, nullptr};   // records of later windows (ping-pong)
   uint32_t defer_cap = 0;
   int defer_cur = 0;
-  uint64_t deferred_last = 0;
 
   uint64_t events_in = 0, pending_since_fold = 0, windows = 0;
   uint64_t launches = 0;                  // own kernels launched (stats)
@@ -99,9 +204,9 @@ struct alz_handle {
   uint64_t tcp_events_in = 0, tcp_localhost_dropped = 0;
 
   int comm_nranks = 1, comm_rank = 0;
-  alz_comm_state* comm = nullptr;
-  alz_gnn_state* gnn = nullptr;
-  alz_sock_state* sock = nullptr;
+  StatePtr<alz_comm_state> comm;          // optional state: published only when complete
+  StatePtr<alz_gnn_state> gnn;
+  StatePtr<alz_sock_state> sock;
 };
 
 int alz_internal_fold(alz_handle* h);
@@ -111,6 +216,3 @@ int alz_internal_ingest(alz_handle* h, const alz_l7_rec* d_recs, size_t n);
 // caller finishes the flush locally. local_rc: this rank's own status so far (every rank enters the
 // collectives even when its local preparation failed, and all ranks return the same failure)
 int alz_internal_merge_ranks(alz_handle* h, int local_rc);
-void alz_internal_free_comm(alz_handle* h);
-void alz_internal_free_gnn(alz_handle* h);
-void alz_internal_free_sock(alz_handle* h);

@@ -240,42 +240,32 @@ using LineMap = std::unordered_map<LineKey, Line, LineKeyHash>;
 }  // namespace
 
 struct alz_sock_state {
+  Owned mem;                                 // ev_stage, d_joined, d_alive_n
   LineMap lines;
   std::vector<LineMap::value_type*> dirty;   // lines with pending ops (node addresses are stable)
   std::vector<LineEnt> h_index;              // host mirror of the index (keys and slots only)
-  LineEnt* d_index = nullptr;
+  GrowBuf<LineEnt> d_index;
   uint32_t index_cap = 0;
-  SockRec* d_pool = nullptr;
+  Owner d_pool;
   size_t pool_cap = 0, pool_used = 0, pool_garbage = 0;
-  void* h_stage = nullptr;                   // pinned: descs then ops of one sync
-  void* d_stage = nullptr;
-  size_t stage_cap = 0;
+  GrowBuf<char> h_stage{Res::kPinned};      // descs then ops of one sync
+  GrowBuf<char> d_stage;
   cudaEvent_t ev_stage = nullptr;            // the H2D out of h_stage is done
-  alz_sock_query* d_q = nullptr;
-  alz_sock_result* d_out = nullptr;
-  size_t q_cap = 0;
-  alz_l7_rec* d_jrec = nullptr;              // alz_submit_l7_join scratch
-  alz_sock_query* d_jkey = nullptr;
-  size_t j_cap = 0;
+  GrowBuf<alz_sock_query> d_q;
+  GrowBuf<alz_sock_result> d_out;
+  GrowBuf<alz_l7_rec> d_jrec;                // alz_submit_l7_join scratch
+  GrowBuf<alz_sock_query> d_jkey;
   unsigned long long* d_joined = nullptr;
-  alz_alive_conn* d_alive = nullptr;
-  size_t alive_cap = 0;
+  GrowBuf<alz_alive_conn> d_alive;
   uint32_t* d_alive_n = nullptr;
   uint64_t syncs = 0, sync_ops = 0, sync_bytes = 0, repools = 0;
+  SockRec* pool() const { return static_cast<SockRec*>(d_pool.get()); }
 };
-
-#define CK(expr)                                                                       \
-  do {                                                                                 \
-    cudaError_t _e = (expr);                                                           \
-    if (_e != cudaSuccess) {                                                           \
-      h->last_err = std::string(#expr) + ": " + cudaGetErrorString(_e);                \
-      return ALZ_E_CUDA;                                                               \
-    }                                                                                  \
-  } while (0)
+void StateDelete::operator()(alz_sock_state* s) const { delete s; }
 
 static alz_sock_state* state_of(alz_handle* h) {
-  if (!h->sock) h->sock = new alz_sock_state();
-  return h->sock;
+  if (!h->sock) h->sock.reset(new alz_sock_state());
+  return h->sock.get();
 }
 
 static void enqueue(alz_sock_state* s, LineMap::value_type* node) {
@@ -358,10 +348,10 @@ static uint32_t seg_cap_for(size_t len) { return std::max<uint32_t>(8u, pow2_at_
 // since the last sync (the apply kernel shifts and moves on the device); the index is re-sent whole only
 // when it doubles, the pool is re-laid only when it is full or half garbage.
 static int sync_lines(alz_handle* h) {
-  alz_sock_state* s = h->sock;
+  alz_sock_state* s = h->sock.get();
   if (s->dirty.empty()) return ALZ_OK;
-  if (!s->ev_stage) CK(cudaEventCreateWithFlags(&s->ev_stage, cudaEventDisableTiming));
-  if (!s->d_joined) { CK(cudaMalloc(&s->d_joined, 8)); CK(cudaMemsetAsync(s->d_joined, 0, 8, h->stream)); }
+  if (!s->ev_stage) CK(s->mem.event(&s->ev_stage, cudaEventDisableTiming));
+  if (!s->d_joined) { CK(s->mem.dev(&s->d_joined, 8)); CK(cudaMemsetAsync(s->d_joined, 0, 8, h->stream)); }
 
   // 1. index: a slot for every new line; doubling rebuilds the mirror and re-sends it
   bool index_resend = false;
@@ -376,9 +366,7 @@ static int sync_lines(alz_handle* h) {
       e.used = 1; e.pid = kv.first.pid; e.fd = kv.first.fd; e.off = L.off; e.len = L.dev_len;
       L.slot = slot;
     }
-    cudaFree(s->d_index);
-    s->d_index = nullptr;
-    CK(cudaMalloc(&s->d_index, (size_t)cap * sizeof(LineEnt)));
+    CK(s->d_index.ensure(cap, h->stream));
     s->index_cap = cap;
     index_resend = true;
   } else {
@@ -401,7 +389,7 @@ static int sync_lines(alz_handle* h) {
   }
   const bool repool = s->pool_used + need > s->pool_cap ||
                       (s->pool_garbage > (1u << 16) && s->pool_garbage * 2 > s->pool_used);
-  SockRec* src_pool = s->d_pool;
+  Owner old_pool;   // a repool's source: freed on return, after the apply kernel has read it
   std::vector<LineDesc> descs;
   std::vector<LineOp> ops;
   auto add_desc = [&](LineMap::value_type* node, uint32_t src_off) {
@@ -420,10 +408,11 @@ static int sync_lines(alz_handle* h) {
     size_t total = 0;
     for (auto& kv : s->lines) total += seg_cap_for(kv.second.v.size());
     const size_t cap = std::max<size_t>(1u << 16, total * 2);
-    if (cap > 0xFFFFFFF0ull) { h->last_err = "socket timelines: more than 2^32 records"; return ALZ_E_CAPACITY; }
-    SockRec* fresh = nullptr;
-    CK(cudaMalloc(&fresh, cap * sizeof(SockRec)));
-    s->d_pool = fresh; s->pool_cap = cap; s->pool_used = 0; s->pool_garbage = 0;
+    if (cap > 0xFFFFFFF0ull) return alz_error(h, ALZ_E_CAPACITY, "socket timelines", "more than 2^32 records");
+    Owner fresh;
+    CK(alz_alloc(fresh, Res::kDev, cap * sizeof(SockRec)));
+    old_pool = std::move(s->d_pool);
+    s->d_pool = std::move(fresh); s->pool_cap = cap; s->pool_used = 0; s->pool_garbage = 0;
     for (auto& kv : s->lines) {                                        // every line moves, on the device
       Line& L = kv.second;
       const uint32_t old_off = L.off;
@@ -451,31 +440,27 @@ static int sync_lines(alz_handle* h) {
   // 3. one staged copy, one kernel
   const size_t desc_bytes = (descs.size() * sizeof(LineDesc) + 15u) & ~(size_t)15u;
   const size_t bytes = desc_bytes + ops.size() * sizeof(LineOp);
-  if (bytes > s->stage_cap) {
-    if (s->h_stage) { CK(cudaEventSynchronize(s->ev_stage)); cudaFreeHost(s->h_stage); s->h_stage = nullptr; }
-    if (s->d_stage) { CK(cudaStreamSynchronize(h->stream)); cudaFree(s->d_stage); s->d_stage = nullptr; }
-    s->stage_cap = bytes * 2;
-    CK(cudaMallocHost(&s->h_stage, s->stage_cap));
-    CK(cudaMalloc(&s->d_stage, s->stage_cap));
-  }
+  CK(s->h_stage.ensure(bytes, h->stream, bytes * 2));
+  CK(s->d_stage.ensure(bytes, h->stream, bytes * 2));
   CK(cudaEventSynchronize(s->ev_stage));
-  memcpy(s->h_stage, descs.data(), descs.size() * sizeof(LineDesc));
-  if (!ops.empty()) memcpy((char*)s->h_stage + desc_bytes, ops.data(), ops.size() * sizeof(LineOp));
+  char* stage = s->h_stage.get();
+  memcpy(stage, descs.data(), descs.size() * sizeof(LineDesc));
+  if (!ops.empty()) memcpy(stage + desc_bytes, ops.data(), ops.size() * sizeof(LineOp));
   if (index_resend)
-    CK(cudaMemcpyAsync(s->d_index, s->h_index.data(), (size_t)s->index_cap * sizeof(LineEnt), cudaMemcpyHostToDevice,
+    CK(cudaMemcpyAsync(s->d_index.get(), s->h_index.data(), (size_t)s->index_cap * sizeof(LineEnt), cudaMemcpyHostToDevice,
                        h->stream));
-  CK(cudaMemcpyAsync(s->d_stage, s->h_stage, bytes, cudaMemcpyHostToDevice, h->stream));
+  CK(cudaMemcpyAsync(s->d_stage.get(), stage, bytes, cudaMemcpyHostToDevice, h->stream));
   CK(cudaEventRecord(s->ev_stage, h->stream));
   const unsigned blocks = (unsigned)std::min<size_t>((descs.size() + 3) / 4, (size_t)h->sms * 8);
   sock_apply_kernel<<<std::max(1u, blocks), 128, 0, h->stream>>>(
-      src_pool ? src_pool : s->d_pool, s->d_pool, s->d_index, (const LineDesc*)s->d_stage,
-      (const LineOp*)((const char*)s->d_stage + desc_bytes), (uint32_t)descs.size());
+      old_pool ? static_cast<SockRec*>(old_pool.get()) : s->pool(), s->pool(), s->d_index.get(),
+      (const LineDesc*)s->d_stage.get(), (const LineOp*)(s->d_stage.get() + desc_bytes), (uint32_t)descs.size());
   CK(cudaGetLastError());
   h->launches++;
   s->syncs++; s->sync_ops += ops.size();
   s->sync_bytes += bytes + (index_resend ? (size_t)s->index_cap * sizeof(LineEnt) : 0);
   if (index_resend) CK(cudaStreamSynchronize(h->stream));   // h_index is pageable
-  if (repool && src_pool) { CK(cudaStreamSynchronize(h->stream)); cudaFree(src_pool); }
+  if (old_pool) CK(cudaStreamSynchronize(h->stream));
   return ALZ_OK;
 }
 
@@ -496,21 +481,14 @@ extern "C" int alz_sock_lookup_at(alz_handle* h, const alz_sock_query* q, size_t
   int rc = sync_lines(h);
   if (rc != ALZ_OK) return rc;
   if (s->index_cap == 0) { memset(out, 0, n * sizeof(alz_sock_result)); return ALZ_OK; }   // no line yet
-  if (n > s->q_cap) {
-    CK(cudaStreamSynchronize(h->stream));
-    cudaFree(s->d_q); cudaFree(s->d_out);
-    s->d_q = nullptr; s->d_out = nullptr;
-    s->q_cap = 0;
-    CK(cudaMalloc(&s->d_q, n * sizeof(alz_sock_query)));
-    CK(cudaMalloc(&s->d_out, n * sizeof(alz_sock_result)));
-    s->q_cap = n;
-  }
-  CK(cudaMemcpyAsync(s->d_q, q, n * sizeof(alz_sock_query), cudaMemcpyHostToDevice, h->stream));
-  sock_lookup_kernel<<<(unsigned)h->sms * 4, 256, 0, h->stream>>>(s->d_index, s->index_cap - 1, s->d_pool, s->d_q,
-                                                                (uint32_t)n, now_ns, s->d_out);
+  CK(s->d_q.ensure(n, h->stream));
+  CK(s->d_out.ensure(n, h->stream));
+  CK(cudaMemcpyAsync(s->d_q.get(), q, n * sizeof(alz_sock_query), cudaMemcpyHostToDevice, h->stream));
+  sock_lookup_kernel<<<(unsigned)h->sms * 4, 256, 0, h->stream>>>(s->d_index.get(), s->index_cap - 1, s->pool(),
+                                                                s->d_q.get(), (uint32_t)n, now_ns, s->d_out.get());
   CK(cudaGetLastError());
   h->launches++;
-  CK(cudaMemcpyAsync(out, s->d_out, n * sizeof(alz_sock_result), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(out, s->d_out.get(), n * sizeof(alz_sock_result), cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   return ALZ_OK;
 }
@@ -530,28 +508,23 @@ extern "C" int alz_submit_l7_join(alz_handle* h, const alz_l7_rec* recs, const a
   alz_sock_state* s = state_of(h);
   int rc = sync_lines(h);
   if (rc != ALZ_OK) return rc;
-  if (!s->d_joined) { CK(cudaMalloc(&s->d_joined, 8)); CK(cudaMemsetAsync(s->d_joined, 0, 8, h->stream)); }
+  if (!s->d_joined) { CK(s->mem.dev(&s->d_joined, 8)); CK(cudaMemsetAsync(s->d_joined, 0, 8, h->stream)); }
   const size_t per = h->cfg.max_batch;
-  if (per > s->j_cap) {
-    CK(cudaStreamSynchronize(h->stream));
-    cudaFree(s->d_jrec); cudaFree(s->d_jkey);
-    s->d_jrec = nullptr; s->d_jkey = nullptr; s->j_cap = 0;
-    CK(cudaMalloc(&s->d_jrec, per * sizeof(alz_l7_rec)));
-    CK(cudaMalloc(&s->d_jkey, per * sizeof(alz_sock_query)));
-    s->j_cap = per;
-  }
+  CK(s->d_jrec.ensure(per, h->stream));
+  CK(s->d_jkey.ensure(per, h->stream));
   if (now_ns == 0) now_ns = wall_ns();
   for (size_t done = 0; done < n; done += per) {
     const size_t m = std::min(per, n - done);
-    CK(cudaMemcpyAsync(s->d_jrec, recs + done, m * sizeof(alz_l7_rec), cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemcpyAsync(s->d_jkey, keys + done, m * sizeof(alz_sock_query), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(s->d_jrec.get(), recs + done, m * sizeof(alz_l7_rec), cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(s->d_jkey.get(), keys + done, m * sizeof(alz_sock_query), cudaMemcpyHostToDevice, h->stream));
     if (s->index_cap != 0) {
-      sock_join_kernel<<<(unsigned)h->sms * 4, 256, 0, h->stream>>>(s->d_index, s->index_cap - 1, s->d_pool, s->d_jkey,
-                                                                  (uint32_t)m, now_ns, s->d_jrec, s->d_joined);
+      sock_join_kernel<<<(unsigned)h->sms * 4, 256, 0, h->stream>>>(s->d_index.get(), s->index_cap - 1, s->pool(),
+                                                                  s->d_jkey.get(), (uint32_t)m, now_ns, s->d_jrec.get(),
+                                                                  s->d_joined);
       CK(cudaGetLastError());
       h->launches++;
     }
-    rc = alz_internal_ingest(h, s->d_jrec, m);
+    rc = alz_internal_ingest(h, s->d_jrec.get(), m);
     if (rc != ALZ_OK) return rc;
     CK(cudaStreamSynchronize(h->stream));   // one scratch buffer; the caller's arrays may be pageable
   }
@@ -592,7 +565,7 @@ extern "C" int alz_sock_gc(alz_handle* h) {
   if (rc != ALZ_OK) return rc;
   if (s->pool_used == 0) return ALZ_OK;
   std::vector<SockRec> pool(s->pool_used);
-  CK(cudaMemcpyAsync(pool.data(), s->d_pool, s->pool_used * sizeof(SockRec), cudaMemcpyDeviceToHost, h->stream));
+  CK(cudaMemcpyAsync(pool.data(), s->pool(), s->pool_used * sizeof(SockRec), cudaMemcpyDeviceToHost, h->stream));
   CK(cudaStreamSynchronize(h->stream));
   for (auto& kv : s->lines) {
     Line& L = kv.second;
@@ -621,17 +594,11 @@ extern "C" int alz_sock_alive(alz_handle* h, alz_alive_conn* out, size_t cap, si
   if (rc != ALZ_OK) return rc;
   *n_out = 0;
   if (s->index_cap == 0) return ALZ_OK;
-  if (!s->d_alive_n) CK(cudaMalloc(&s->d_alive_n, 4));
-  if (cap > s->alive_cap) {
-    CK(cudaStreamSynchronize(h->stream));
-    cudaFree(s->d_alive);
-    s->d_alive = nullptr; s->alive_cap = 0;
-    CK(cudaMalloc(&s->d_alive, cap * sizeof(alz_alive_conn)));
-    s->alive_cap = cap;
-  }
+  if (!s->d_alive_n) CK(s->mem.dev(&s->d_alive_n, 4));
+  CK(s->d_alive.ensure(cap, h->stream));
   CK(cudaMemsetAsync(s->d_alive_n, 0, 4, h->stream));
-  sock_alive_kernel<<<(unsigned)h->sms * 4, 256, 0, h->stream>>>(s->d_index, s->index_cap, s->d_pool, h->d_ep,
-                                                               h->ep_cap - 1, s->d_alive,
+  sock_alive_kernel<<<(unsigned)h->sms * 4, 256, 0, h->stream>>>(s->d_index.get(), s->index_cap, s->pool(), h->d_ep,
+                                                               h->ep_cap - 1, s->d_alive.get(),
                                                                (uint32_t)std::min<size_t>(cap, 0xFFFFFFFFu), s->d_alive_n);
   CK(cudaGetLastError());
   h->launches++;
@@ -640,7 +607,7 @@ extern "C" int alz_sock_alive(alz_handle* h, alz_alive_conn* out, size_t cap, si
   CK(cudaStreamSynchronize(h->stream));
   *n_out = cnt;                                                          // the number there are
   const size_t take = std::min<size_t>(cnt, cap);
-  if (take) CK(cudaMemcpy(out, s->d_alive, take * sizeof(alz_alive_conn), cudaMemcpyDeviceToHost));
+  if (take) CK(cudaMemcpy(out, s->d_alive.get(), take * sizeof(alz_alive_conn), cudaMemcpyDeviceToHost));
   return cnt > cap ? ALZ_E_CAPACITY : ALZ_OK;
 }
 
@@ -648,7 +615,7 @@ extern "C" int alz_sock_stats(alz_handle* h, alz_sock_stats_t* st) {
   if (!h || !st) return ALZ_E_INVAL;
   std::lock_guard<std::mutex> g(h->mu);
   memset(st, 0, sizeof *st);
-  alz_sock_state* s = h->sock;
+  alz_sock_state* s = h->sock.get();
   if (!s) return ALZ_OK;
   CK(cudaSetDevice(h->device));
   st->lines = s->lines.size();
@@ -665,16 +632,4 @@ extern "C" int alz_sock_stats(alz_handle* h, alz_sock_stats_t* st) {
     st->joined_events = j;
   }
   return ALZ_OK;
-}
-
-void alz_internal_free_sock(alz_handle* h) {
-  alz_sock_state* s = h->sock;
-  if (!s) return;
-  cudaFree(s->d_index); cudaFree(s->d_pool); cudaFree(s->d_q); cudaFree(s->d_out);
-  cudaFree(s->d_stage); cudaFree(s->d_jrec); cudaFree(s->d_jkey); cudaFree(s->d_joined);
-  cudaFree(s->d_alive); cudaFree(s->d_alive_n);
-  if (s->h_stage) cudaFreeHost(s->h_stage);
-  if (s->ev_stage) cudaEventDestroy(s->ev_stage);
-  delete s;
-  h->sock = nullptr;
 }
