@@ -68,6 +68,7 @@ def load(rebuild=False):
         "alz_gnn_score": ([vp, vp, sz, C.POINTER(sz)], i),
         "alz_gnn_score_device": ([vp, pp, C.POINTER(sz)], i),
         "alz_gnn_nodes": ([vp, vp, vp, sz, C.POINTER(sz)], i),
+        "alz_merge_blocks_device": ([vp, vp, u32, u32, pp, C.POINTER(sz)], i),
         "alz_edge_quantiles": ([vp, vp, sz, vp], i),
         "alz_submit_tcp": ([vp, vp, sz], i),
         "alz_sock_lookup": ([vp, vp, sz, vp], i),

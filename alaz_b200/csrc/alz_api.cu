@@ -185,10 +185,8 @@ extern "C" int alz_create(const alz_config* cfg, alz_handle** out) {
   if ((rc = alloc_table(h, &h->edges, h->cfg.max_edges, &h->d_ctr->edge_rows, false)) != ALZ_OK) return fail(rc);
   CKC(m.pinned(&h->h_ctr, sizeof(Counters)));
   memset(h->h_ctr, 0, sizeof(Counters));
-  for (int b = 0; b < 2; ++b) {
-    CKC(m.dev(&h->d_keys[b], (size_t)h->cfg.max_edges * 8));
-    CKC(m.dev(&h->d_rows[b], (size_t)h->cfg.max_edges * 4));
-  }
+  CKC(m.dev(&h->d_keys, (size_t)h->cfg.max_edges * 8));
+  for (int b = 0; b < 2; ++b) CKC(m.dev(&h->d_rows[b], (size_t)h->cfg.max_edges * 4));
   h->sort_tmp_bytes = sort_pairs_temp_bytes(h->cfg.max_edges);
   CKC(m.dev(&h->d_sort_tmp, h->sort_tmp_bytes));
   CKC(m.dev(&h->d_out, (size_t)h->cfg.max_edges * sizeof(alz_edge_out)));
@@ -622,7 +620,7 @@ extern "C" int alz_submit_l7_raw(alz_handle* h, const void* raw, size_t n) {
 }
 
 // ---- window result ---------------------------------------------------------------------------
-// Fold + sort of the live edge keys (no reset). After it h->n_live edges sit in d_keys[1]/d_rows[1].
+// Fold + sort of the live edge keys (no reset). After it h->n_live edges sit in d_keys/d_rows[1].
 // The edge count is final once the first half of the fold has run, so the counters are copied out right
 // there and the host waits on an event for THAT copy only: the second half of the fold is still
 // running on the GPU while the host sizes and enqueues the sort (r1 stalled the whole stream here).
@@ -643,7 +641,7 @@ static int prepare_flush(alz_handle* h, bool* overflow) {
   if (h->n_live) {
     launch_iota(h->d_rows[0], h->n_live, h->sms, h->stream);
     h->launches += 1;
-    sort_pairs(h->d_sort_tmp, h->sort_tmp_bytes, h->edges.row_key, h->d_keys[1], h->d_rows[0], h->d_rows[1],
+    sort_pairs(h->d_sort_tmp, h->sort_tmp_bytes, h->edges.row_key, h->d_keys, h->d_rows[0], h->d_rows[1],
                h->n_live, h->stream);
     CK(cudaGetLastError());
   }
@@ -651,7 +649,7 @@ static int prepare_flush(alz_handle* h, bool* overflow) {
 }
 
 static int finish_flush(alz_handle* h) {
-  launch_gather_edges(h->edges, h->d_keys[1], h->d_rows[1], h->n_live, h->d_out, true, h->sms, h->stream);
+  launch_gather_edges(h->edges, h->d_keys, h->d_rows[1], h->n_live, h->d_out, true, h->sms, h->stream);
   h->launches += h->n_live ? 1 : 0;
   CK(cudaGetLastError());
   int rc = clear_dict(h, &h->edges);
@@ -684,8 +682,10 @@ static int flush_device_locked(alz_handle* h, const alz_edge_out** dev_edges, si
   int rc = prepare_flush(h, &overflow);
   *n_out = h->n_live;
   CK(cudaEventRecord(h->ev_t[1], h->stream));
-  int mrc = alz_internal_merge_ranks(h, rc);  // multi-GPU: one collective over the ranks' edge rows (alz_comm.cu)
-  if (mrc == ALZ_E_UNSUPPORTED) {             // single rank
+  int mrc;
+  if (h->comm_nranks > 1) {
+    mrc = alz_internal_merge_ranks(h, rc);  // one collective over the ranks' edge rows (alz_comm.cu)
+  } else {
     if (rc != ALZ_OK) return rc;
     mrc = finish_flush(h);
   }

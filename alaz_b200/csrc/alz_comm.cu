@@ -3,7 +3,7 @@
 // reaches one rank, so the ranks' edge sets are disjoint and a rank's accumulators are
 // already final: what the flush has to do is hand every rank every other rank's rows.
 //
-// Default path — ONE collective, no host round trip before it:
+// ONE collective, no host round trip before it:
 //   1. each rank writes its sorted live rows behind a one-row header {count, status} in a
 //      send buffer; the per-rank block size of the collective comes from the previous
 //      window's counts (+25 %), so no count exchange is needed
@@ -18,9 +18,10 @@
 // A block that was too small (traffic grew by more than 25 % in one window) is sent
 // again, larger; the local rows are only reset after a successful merge.
 //
-// General path (a key present on several ranks: the caller did not partition by
-// alz_owner_rank): canonical dictionary by all-gather + sort + unique, local rows
-// scattered into a zeroed canonical array, ONE ncclAllReduce(sum) on the accumulators.
+// Overlapping ranks (a key present on several ranks: the caller did not partition by
+// alz_owner_rank): after the all-gather every rank holds every rank's complete rows, the
+// same bytes on every rank, so each rank merges them locally with no further exchange:
+// sort the live rows by key, then one row per distinct key with the sums of its rows.
 // Integer sums either way, so bit-exact for any rank count.
 //
 // NCCL is loaded lazily with dlopen so that single-GPU users (and the Go agent
@@ -29,6 +30,7 @@
 #include <nccl.h>
 
 #include <algorithm>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <mutex>
@@ -46,7 +48,6 @@ struct NcclApi {
   ncclResult_t (*CommInitRank)(ncclComm_t*, int, ncclUniqueId, int) = nullptr;
   ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
   ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
-  ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
   const char* (*GetErrorString)(ncclResult_t) = nullptr;
 };
 NcclApi g_nccl;
@@ -62,7 +63,6 @@ bool load_nccl_once() {
   SYM(CommInitRank, "ncclCommInitRank");
   SYM(CommDestroy, "ncclCommDestroy");
   SYM(AllGather, "ncclAllGather");
-  SYM(AllReduce, "ncclAllReduce");
   SYM(GetErrorString, "ncclGetErrorString");
 #undef SYM
   g_nccl.lib = lib;
@@ -76,115 +76,30 @@ bool load_nccl() {
   return ok;
 }
 
-constexpr int kCanWords = 3 + ALZ_NB;      // u64 words per canonical edge row of the general path: count, err5xx,
-                                           // lat_sum and one word per histogram cell (a cell is u32 modulo 2^32: the
-                                           // low halves of the sums are taken, nothing can carry between cells)
+constexpr uint32_t kMaxRanks = 64;                     // merge_blocks_kernel keeps one count per rank in shared memory
 constexpr uint32_t kRowBytes = sizeof(alz_edge_out);   // 296 = 37 x 8
 constexpr uint32_t kRowWords64 = kRowBytes / 8;
+constexpr uint32_t kSumWord = offsetof(alz_edge_out, count) / 8;   // words [kSumWord, kHistWord): u64 sums
+constexpr uint32_t kHistWord = offsetof(alz_edge_out, hist) / 8;   // words from kHistWord on: two u32 cells each
+static_assert(offsetof(alz_edge_out, lat_sum_ns) + 8 == offsetof(alz_edge_out, hist) && kHistWord * 8 ==
+              offsetof(alz_edge_out, hist), "alz_edge_out layout");
 constexpr uint32_t kHdrMagic = 0xA1A2C0DEu;
 struct BlockHeader {      // first row of a rank's block
   uint32_t magic, count;
   int32_t status;
   uint32_t pad;
 };
-struct MergeInfo {        // written by the merge kernel, read by the host
+struct MergeInfo {        // written by the merge kernels, read by the host
   uint32_t total, dup, overflow, max_count;
   int32_t peer_status;
-  uint32_t pad[3];
+  uint32_t n_unique;      // overlapping ranks: rows after the merge
+  uint32_t pad[2];
 };
-
-// out[i] = keys[i] for i < n, kEmptyKey padding up to n_pad
-__global__ void pad_keys_kernel(const uint64_t* __restrict__ keys, uint32_t n, uint64_t* __restrict__ out,
-                                uint32_t n_pad) {
-  const uint32_t stride = gridDim.x * blockDim.x;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_pad; i += stride)
-    out[i] = i < n ? keys[i] : kEmptyKey;
-}
-
-// unique of the sorted gathered keys: flag run heads, exclusive-scan the flags, scatter the heads
-__global__ void flag_heads_kernel(const uint64_t* __restrict__ sorted, uint32_t n, uint32_t* __restrict__ flags) {
-  const uint32_t stride = gridDim.x * blockDim.x;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-    const uint64_t k = sorted[i];
-    flags[i] = (k != kEmptyKey && (i == 0 || sorted[i - 1] != k)) ? 1u : 0u;
-  }
-}
-__global__ void scatter_heads_kernel(const uint64_t* __restrict__ sorted, const uint32_t* __restrict__ flags,
-                                     const uint32_t* __restrict__ pos, uint32_t n, uint64_t* __restrict__ out) {
-  const uint32_t stride = gridDim.x * blockDim.x;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
-    if (flags[i]) out[pos[i]] = sorted[i];
-}
 
 __device__ __forceinline__ uint32_t lower_bound_u64(const uint64_t* __restrict__ a, uint32_t n, uint64_t k) {
   uint32_t lo = 0, hi = n;
   while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (a[mid] < k) lo = mid + 1; else hi = mid; }
   return lo;
-}
-
-// union of R sorted, pairwise disjoint key lists (segment r = gathered[r * pad .. + counts[r])):
-// out[sum of lower bounds] = key. *dup is set if a key occurs in two lists.
-__global__ void __launch_bounds__(256) merge_disjoint_kernel(const uint64_t* __restrict__ gathered, uint32_t pad,
-                                                             uint32_t R, const uint32_t* __restrict__ counts,
-                                                             uint64_t* __restrict__ out, uint32_t* __restrict__ dup) {
-  const uint32_t stride = gridDim.x * blockDim.x;
-  for (uint32_t t = blockIdx.x * blockDim.x + threadIdx.x; t < pad * R; t += stride) {
-    const uint32_t r = t / pad, i = t - r * pad;
-    if (i >= counts[r]) continue;
-    const uint64_t k = gathered[t];
-    uint32_t pos = i;
-    for (uint32_t q = 0; q < R; ++q) {
-      if (q == r) continue;
-      const uint64_t* seg = gathered + (size_t)q * pad;
-      const uint32_t lb = lower_bound_u64(seg, counts[q], k);
-      if (lb < counts[q] && seg[lb] == k) *dup = 1u;
-      pos += lb;
-    }
-    out[pos] = k;
-  }
-}
-
-// local live rows -> canonical array (zeroed beforehand); a warp per local edge; rows are zeroed
-__global__ void __launch_bounds__(256) scatter_canonical_kernel(AccTable edges, const uint64_t* __restrict__ keys,
-                                                                const uint32_t* __restrict__ rows, uint32_t n_local,
-                                                                const uint64_t* __restrict__ can_keys, uint32_t n_can,
-                                                                uint64_t* __restrict__ can) {
-  const uint32_t lane = threadIdx.x & 31u;
-  const uint32_t warps_per_grid = (gridDim.x * blockDim.x) >> 5;
-  for (uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n_local; i += warps_per_grid) {
-    const uint32_t row = rows[i];
-    const uint32_t pos = lower_bound_u64(can_keys, n_can, keys[i]);   // always present
-    uint64_t* dst = can + (size_t)pos * kCanWords;
-    dst[3 + lane] = edges.hist[(size_t)row * ALZ_NB + lane];
-    dst[3 + 32 + lane] = edges.hist[(size_t)row * ALZ_NB + 32 + lane];
-    edges.hist[(size_t)row * ALZ_NB + lane] = 0u;
-    edges.hist[(size_t)row * ALZ_NB + 32 + lane] = 0u;
-    if (lane == 0) {
-      dst[0] = edges.count[row]; dst[1] = edges.err5xx[row]; dst[2] = edges.lat_sum[row];
-      edges.count[row] = 0ull; edges.err5xx[row] = 0ull; edges.lat_sum[row] = 0ull;
-    }
-  }
-}
-
-__global__ void __launch_bounds__(256) unpack_canonical_kernel(const uint64_t* __restrict__ can_keys,
-                                                               const uint64_t* __restrict__ can, uint32_t n_can,
-                                                               alz_edge_out* __restrict__ out) {
-  const uint32_t lane = threadIdx.x & 31u;
-  const uint32_t warps_per_grid = (gridDim.x * blockDim.x) >> 5;
-  for (uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n_can; i += warps_per_grid) {
-    const uint64_t* src = can + (size_t)i * kCanWords;
-    alz_edge_out* o = &out[i];
-    o->hist[lane] = (uint32_t)src[3 + lane];
-    o->hist[32 + lane] = (uint32_t)src[3 + 32 + lane];
-    if (lane == 0) {
-      uint8_t ft, tt; uint32_t f, t;
-      unpack_edge_key(can_keys[i], &ft, &f, &tt, &t);
-      o->from_type = ft; o->to_type = tt;
-      for (int k = 0; k < 6; ++k) o->_pad[k] = 0;
-      o->from = f; o->to = t;
-      o->count = src[0]; o->err5xx = src[1]; o->lat_sum_ns = src[2];
-    }
-  }
 }
 
 // packed edge key of an output row (inverse of unpack_edge_key)
@@ -208,7 +123,7 @@ __device__ __forceinline__ uint32_t lower_bound_rows(const alz_edge_out* rows, u
 __global__ void __launch_bounds__(256) merge_blocks_kernel(const alz_edge_out* __restrict__ recv, uint32_t cap, uint32_t R,
                                                            alz_edge_out* __restrict__ out, uint32_t out_cap,
                                                            MergeInfo* __restrict__ info) {
-  __shared__ uint32_t s_cnt[64];
+  __shared__ uint32_t s_cnt[kMaxRanks];
   __shared__ uint32_t s_bad;
   const size_t stride_rows = (size_t)cap + 1;
   if (threadIdx.x == 0) s_bad = 0u;
@@ -260,12 +175,13 @@ __global__ void __launch_bounds__(256) merge_blocks_kernel(const alz_edge_out* _
   }
 }
 
-// a successful merge consumes the window: zero the local edge rows that were sent, empty the edge dictionary, reset
-// the row allocator. Decided on the device from the merge kernel's verdict, so the host reads that verdict once, at
-// the end, instead of synchronising in the middle of the flush to decide whether to launch this.
+// a merge without a failed peer or an overflow consumes the window: zero the local edge rows that were sent, empty
+// the edge dictionary, reset the row allocator. Decided on the device from the merge kernel's verdict, so the host
+// reads that verdict once, at the end, instead of synchronising in the middle of the flush to decide whether to
+// launch this. Overlapping ranks are merged from the gathered blocks alone, so they consume the window too.
 __global__ void __launch_bounds__(256) consume_window_kernel(const MergeInfo* __restrict__ info, AccTable edges,
                                                              const uint32_t* __restrict__ rows, uint32_t n) {
-  if (info->peer_status != ALZ_OK || info->overflow != 0u || info->dup != 0u) return;
+  if (info->peer_status != ALZ_OK || info->overflow != 0u) return;
   const uint32_t sl = threadIdx.x & 7u;
   const uint32_t groups = (gridDim.x * blockDim.x) >> 3;
   const size_t dict_words = ((size_t)edges.dict_mask + 1u) * (sizeof(DictEnt) / 16u);
@@ -282,32 +198,74 @@ __global__ void __launch_bounds__(256) consume_window_kernel(const MergeInfo* __
   }
 }
 
+// overlapping ranks: packed key and index in recv of every live row of the gathered blocks, in block order
+__global__ void __launch_bounds__(256) live_row_keys_kernel(const alz_edge_out* __restrict__ recv, uint32_t cap,
+                                                            uint32_t R, uint32_t total, uint64_t* __restrict__ keys,
+                                                            uint32_t* __restrict__ rows) {
+  __shared__ uint32_t s_cnt[kMaxRanks];
+  const size_t stride_rows = (size_t)cap + 1;
+  if (threadIdx.x < R) s_cnt[threadIdx.x] = reinterpret_cast<const BlockHeader*>(recv + threadIdx.x * stride_rows)->count;
+  __syncthreads();
+  const uint32_t stride = gridDim.x * blockDim.x;
+  for (uint32_t g = blockIdx.x * blockDim.x + threadIdx.x; g < total; g += stride) {
+    uint32_t q = 0, i = g;
+    while (i >= s_cnt[q]) { i -= s_cnt[q]; ++q; }
+    const uint32_t row = (uint32_t)(q * stride_rows + 1 + i);
+    keys[g] = row_key_of(recv + row);
+    rows[g] = row;
+  }
+}
+
+__device__ __forceinline__ uint64_t add_cells(uint64_t a, uint64_t b) {   // two u32 histogram cells, each modulo 2^32
+  return (uint64_t)((uint32_t)a + (uint32_t)b) | ((uint64_t)((uint32_t)(a >> 32) + (uint32_t)(b >> 32)) << 32);
+}
+
+// overlapping ranks: out[u] = the sum of the gathered rows whose key is ukeys[u]; keys/rows: all live rows, sorted
+// by key. The type and id words come from the run's first row. count, err5xx and lat_sum add modulo 2^64 and each
+// histogram cell modulo 2^32: the bits an element-wise integer sum over the ranks gives. Eight lanes per output row.
+__global__ void __launch_bounds__(256) sum_runs_kernel(const alz_edge_out* __restrict__ recv,
+                                                       const uint64_t* __restrict__ keys,
+                                                       const uint32_t* __restrict__ rows, uint32_t n,
+                                                       const uint64_t* __restrict__ ukeys,
+                                                       const uint32_t* __restrict__ n_unique,
+                                                       alz_edge_out* __restrict__ out) {
+  const uint32_t nu = *n_unique;
+  const uint32_t sl = threadIdx.x & 7u;
+  const uint32_t groups = (gridDim.x * blockDim.x) >> 3;
+  for (uint32_t u = (blockIdx.x * blockDim.x + threadIdx.x) >> 3; u < nu; u += groups) {
+    const uint64_t key = ukeys[u];
+    const uint32_t first = lower_bound_u64(keys, n, key);
+    uint64_t* d64 = reinterpret_cast<uint64_t*>(out + u);
+    for (uint32_t w = sl; w < kRowWords64; w += 8u) {
+      uint64_t v = reinterpret_cast<const uint64_t*>(recv + rows[first])[w];
+      for (uint32_t j = first + 1; w >= kSumWord && j < n && keys[j] == key; ++j) {
+        const uint64_t x = reinterpret_cast<const uint64_t*>(recv + rows[j])[w];
+        v = w < kHistWord ? v + x : add_cells(v, x);
+      }
+      d64[w] = v;
+    }
+  }
+}
+
 }  // namespace
 
 struct alz_comm_state {
   ~alz_comm_state() { if (comm && g_nccl.CommDestroy) g_nccl.CommDestroy(comm); }   // before the buffers below go
   Owned mem;
   ncclComm_t comm = nullptr;
-  uint32_t* d_counts = nullptr;   // [nranks]
+  uint32_t* d_counts = nullptr;   // [nranks]: the first window's count exchange
   uint32_t* h_counts = nullptr;   // pinned
-  uint64_t* d_gather = nullptr;   // [nranks * pad] gathered keys, then sorted copy behind it
-  uint64_t* d_sorted = nullptr;
-  uint32_t* d_flags = nullptr;
-  uint32_t* d_pos = nullptr;
-  uint64_t* d_can_keys = nullptr; // [max_edges]
-  uint64_t* d_can = nullptr;      // [max_edges * kCanWords]
-  uint32_t* d_iota = nullptr;
-  uint32_t* d_vals = nullptr;
-  void* d_tmp = nullptr;
-  size_t tmp_bytes = 0;
-  size_t gather_cap = 0;          // keys
-  // default path
   alz_edge_out* d_send = nullptr; // [1 + block_rows_for(max_edges)]: header row + local sorted rows (+ head room)
   GrowBuf<alz_edge_out> d_recv;   // [R * (1 + cap_r)]
   uint32_t cap_r = 0;             // rows per rank block of the next collective (0 = not known yet)
   BlockHeader* h_hdr = nullptr;   // pinned
   MergeInfo* d_info = nullptr;
   MergeInfo* h_info = nullptr;    // pinned
+  // overlapping ranks only, grown on first use (n = live rows of all blocks): keys [2n] (the rows' keys, then sorted;
+  // the distinct keys overwrite the first half), idx [4n] (row indices, sorted; head flags; unique positions)
+  GrowBuf<uint64_t> ov_keys;
+  GrowBuf<uint32_t> ov_idx;
+  GrowBuf<uint8_t> ov_tmp;
 };
 void StateDelete::operator()(alz_comm_state* c) const { delete c; }
 
@@ -333,8 +291,16 @@ static uint32_t block_rows_for(uint64_t max_count) {   // +25 % head room, in st
   return (uint32_t)((want + 1023) / 1024 * 1024);
 }
 
+// the merge verdict on the device and its pinned copy
+static int alloc_info(alz_handle* h, alz_comm_state* c) {
+  CK(c->mem.dev(&c->d_info, sizeof(MergeInfo)));
+  CK(c->mem.pinned(&c->h_info, sizeof(MergeInfo)));
+  return ALZ_OK;
+}
+
 extern "C" int alz_comm_init(alz_handle* h, int nranks, int rank, const void* id_bytes) {
   if (!h || !id_bytes || nranks < 1 || rank < 0 || rank >= nranks) return ALZ_E_INVAL;
+  if (nranks > (int)kMaxRanks) return ALZ_E_UNSUPPORTED;
   std::lock_guard<std::mutex> g(h->mu);
   if (h->comm) return ALZ_E_STATE;
   if (!load_nccl()) return alz_error(h, ALZ_E_NCCL, nullptr, "dlopen(libnccl.so.2) failed");
@@ -346,116 +312,87 @@ extern "C" int alz_comm_init(alz_handle* h, int nranks, int rank, const void* id
   ncclComm_t comm = nullptr;
   NK(g_nccl.CommInitRank(&comm, nranks, id, rank));
   c->comm = comm;
-  const size_t me = h->cfg.max_edges;
-  c->gather_cap = me;  // every rank holds the merged graph, so max_edges bounds the gathered keys too
   Owned& m = c->mem;
   CK(m.dev(&c->d_counts, sizeof(uint32_t) * nranks));
   CK(m.pinned(&c->h_counts, sizeof(uint32_t) * nranks));
-  CK(m.dev(&c->d_gather, me * 8 * 2));
-  c->d_sorted = c->d_gather + me;
-  CK(m.dev(&c->d_flags, me * 4));
-  CK(m.dev(&c->d_pos, me * 4));
-  CK(m.dev(&c->d_can_keys, me * 8));
-  CK(m.dev(&c->d_can, me * kCanWords * 8));
-  CK(m.dev(&c->d_iota, me * 4));
-  CK(m.dev(&c->d_vals, me * 4));
-  c->tmp_bytes = std::max(sort_pairs_temp_bytes((uint32_t)me), scan_temp_bytes((uint32_t)me));
-  CK(m.dev(&c->d_tmp, c->tmp_bytes));
   // a block is sized from the largest rank's count plus head room: up to block_rows_for(max_edges) rows are SENT
   // from here even when this rank has fewer (max_edges must be the same on every rank)
-  const size_t send_rows = (size_t)block_rows_for(me) + 1;
+  const size_t send_rows = (size_t)block_rows_for(h->cfg.max_edges) + 1;
   CK(m.dev(&c->d_send, send_rows * sizeof(alz_edge_out)));
   CK(cudaMemset(c->d_send, 0, send_rows * sizeof(alz_edge_out)));
   CK(m.pinned(&c->h_hdr, sizeof(alz_edge_out)));
-  CK(m.dev(&c->d_info, sizeof(MergeInfo)));
-  CK(m.pinned(&c->h_info, sizeof(MergeInfo)));
+  const int rc = alloc_info(h, c.get());
+  if (rc != ALZ_OK) return rc;
   h->comm = std::move(c);
   h->comm_nranks = nranks;
   h->comm_rank = rank;
   return ALZ_OK;
 }
 
-// General path: keys may live on several ranks. Local live edges are sorted in d_keys[1] / d_rows[1].
-static int merge_allreduce(alz_handle* h) {
-  alz_comm_state* c = h->comm.get();
-  const int R = h->comm_nranks;
+// Overlapping ranks: all n live rows of the R gathered blocks, sorted by key, summed per key into h->d_out.
+// *n_unique: rows written, read back in this path's one synchronisation.
+static int merge_overlap(alz_handle* h, alz_comm_state* c, const alz_edge_out* recv, uint32_t cap, uint32_t R,
+                         uint32_t n, uint32_t* n_unique) {
   cudaStream_t s = h->stream;
   const unsigned grid = (unsigned)h->sms * 4;
-
-  // 1. counts
-  CK(cudaMemcpyAsync(c->d_counts + h->comm_rank, &h->n_live, 4, cudaMemcpyHostToDevice, s));
-  NK(g_nccl.AllGather(c->d_counts + h->comm_rank, c->d_counts, 1, ncclUint32, c->comm, s));
-  CK(cudaMemcpyAsync(c->h_counts, c->d_counts, 4 * R, cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
-  uint32_t pad = 0;
-  uint64_t total = 0;
-  for (int r = 0; r < R; ++r) { pad = std::max(pad, c->h_counts[r]); total += c->h_counts[r]; }
-  if (total == 0) {
-    h->last_n_edges = 0;
-    h->windows++;
-    CK(cudaMemsetAsync(h->edges.dict, 0xFF, ((size_t)h->edges.dict_mask + 1) * sizeof(DictEnt), s));
-    CK(cudaMemsetAsync(h->edges.n_rows, 0, 4, s));
-    return ALZ_OK;
-  }
-  if ((uint64_t)pad * R > c->gather_cap) return ALZ_E_CAPACITY;
-  const uint32_t n_g = pad * (uint32_t)R;
-
-  // 2. keys: pad, all-gather, merge. Each rank's list is sorted and, when the caller partitioned by
-  //    alz_owner_rank, the lists are disjoint: a key's place in the union is then the sum of its lower
-  //    bounds in the R lists - no sort. A key found on two ranks (caller routed one source to two ranks)
-  //    raises a flag and the general path (sort + unique) runs instead; the sums are right either way.
-  pad_keys_kernel<<<grid, 256, 0, s>>>(h->d_keys[1], h->n_live, c->d_sorted, pad);
-  NK(g_nccl.AllGather(c->d_sorted, c->d_gather, pad, ncclUint64, c->comm, s));
-  CK(cudaMemsetAsync(c->d_flags, 0, 4, s));
-  merge_disjoint_kernel<<<grid, 256, 0, s>>>(c->d_gather, pad, (uint32_t)R, c->d_counts, c->d_can_keys, c->d_flags);
-  uint32_t dup = 0;
-  CK(cudaMemcpyAsync(&dup, c->d_flags, 4, cudaMemcpyDeviceToHost, s));
-  CK(cudaStreamSynchronize(s));
-  uint32_t n_can = (uint32_t)total;
-  if (dup) {
-    launch_iota(c->d_iota, n_g, h->sms, s);
-    sort_pairs(c->d_tmp, c->tmp_bytes, c->d_gather, c->d_sorted, c->d_iota, c->d_vals, n_g, s);
-    flag_heads_kernel<<<grid, 256, 0, s>>>(c->d_sorted, n_g, c->d_flags);
-    exclusive_scan_u32(c->d_tmp, c->tmp_bytes, c->d_flags, c->d_pos, n_g, s);
-    scatter_heads_kernel<<<grid, 256, 0, s>>>(c->d_sorted, c->d_flags, c->d_pos, n_g, c->d_can_keys);
-    uint32_t last[2];
-    CK(cudaMemcpyAsync(&last[0], c->d_pos + (n_g - 1), 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaMemcpyAsync(&last[1], c->d_flags + (n_g - 1), 4, cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
-    n_can = last[0] + last[1];
-  }
-  if (n_can > h->cfg.max_edges) return ALZ_E_CAPACITY;
-
-  // 3. scatter local rows into the zeroed canonical array
-  const size_t can_bytes = (size_t)n_can * kCanWords * 8;
-  CK(cudaMemsetAsync(c->d_can, 0, can_bytes, s));
-  if (h->n_live)
-    scatter_canonical_kernel<<<grid * 2, 256, 0, s>>>(h->edges, h->d_keys[1], h->d_rows[1], h->n_live,
-                                                      c->d_can_keys, n_can, c->d_can);
-  // 4. the single exchange step
-  NK(g_nccl.AllReduce(c->d_can, c->d_can, (size_t)n_can * kCanWords, ncclUint64, ncclSum, c->comm, s));
-  h->collective_bytes_last += can_bytes;
+  const size_t tmp_bytes = std::max(sort_pairs_temp_bytes(n), scan_temp_bytes(n));
+  CK(c->ov_keys.ensure(2 * (size_t)n, s));
+  CK(c->ov_idx.ensure(4 * (size_t)n, s));
+  CK(c->ov_tmp.ensure(tmp_bytes, s));
+  uint64_t* keys = c->ov_keys.get();
+  uint64_t* sorted = keys + n;
+  uint32_t* rows = c->ov_idx.get();
+  uint32_t* rows_sorted = rows + n;
+  live_row_keys_kernel<<<grid, 256, 0, s>>>(recv, cap, R, n, keys, rows);
+  sort_pairs(c->ov_tmp.get(), tmp_bytes, keys, sorted, rows, rows_sorted, n, s);
+  unique_sorted_u64(c->ov_tmp.get(), tmp_bytes, sorted, n, rows + 2 * (size_t)n, rows + 3 * (size_t)n, keys,
+                    &c->d_info->n_unique, h->sms, s);
+  sum_runs_kernel<<<grid, 256, 0, s>>>(recv, sorted, rows_sorted, n, keys, &c->d_info->n_unique, h->d_out);
   h->launches += 5;
-  // 5. unpack; local edge table back to empty
-  unpack_canonical_kernel<<<grid * 2, 256, 0, s>>>(c->d_can_keys, c->d_can, n_can, h->d_out);
   CK(cudaGetLastError());
-  CK(cudaMemsetAsync(h->edges.dict, 0xFF, ((size_t)h->edges.dict_mask + 1) * sizeof(DictEnt), s));
-  CK(cudaMemsetAsync(h->edges.n_rows, 0, 4, s));
-  h->last_n_edges = n_can;
+  CK(cudaMemcpyAsync(&c->h_info->n_unique, &c->d_info->n_unique, 4, cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));
+  *n_unique = c->h_info->n_unique;
+  return ALZ_OK;
+}
+
+// What the flush runs after the all-gather: merge the R blocks of recv (header row + cap rows each) into h->d_out
+// and read the verdict back into *inf. consume: also reset the local window (n_local rows in h->d_rows[1]) unless a
+// peer failed or something overflowed; the caller handles those. Otherwise the window is complete: overlapping
+// blocks go through merge_overlap, and last_n_edges is set.
+static int merge_gathered(alz_handle* h, alz_comm_state* c, const alz_edge_out* recv, uint32_t cap, uint32_t R,
+                          bool consume, uint32_t n_local, MergeInfo* inf) {
+  cudaStream_t s = h->stream;
+  const unsigned grid = (unsigned)h->sms * 4;
+  CK(cudaMemsetAsync(c->d_info, 0, sizeof(MergeInfo), s));
+  merge_blocks_kernel<<<grid, 256, 0, s>>>(recv, cap, R, h->d_out, h->cfg.max_edges, c->d_info);
+  h->launches += 1;
+  if (consume) {
+    consume_window_kernel<<<grid, 256, 0, s>>>(c->d_info, h->edges, h->d_rows[1], n_local);
+    h->launches += 1;
+  }
+  CK(cudaGetLastError());
+  CK(cudaMemcpyAsync(c->h_info, c->d_info, sizeof(MergeInfo), cudaMemcpyDeviceToHost, s));
+  CK(cudaStreamSynchronize(s));   // the flush's one synchronisation: the caller needs the edge count
+  *inf = *c->h_info;
+  if (inf->peer_status != ALZ_OK || inf->overflow != 0u) return ALZ_OK;
+  uint32_t n = inf->total;
+  if (inf->dup) {                 // not partitioned by owner
+    const int rc = merge_overlap(h, c, recv, cap, R, inf->total, &n);
+    if (rc != ALZ_OK) return rc;
+  }
+  h->last_n_edges = n;
   h->windows++;
   return ALZ_OK;
 }
 
-// Called by the flush after prepare_flush(): local live edges are sorted in d_keys[1] (keys) / d_rows[1]
+// Called by the flush after prepare_flush(): local live edges are sorted in d_keys (keys) / d_rows[1]
 // (rows), h->n_live of them; local_rc is this rank's status so far. Every rank enters the collective whatever
 // its own status, so nobody is left waiting in NCCL, and all ranks return the same failure.
 int alz_internal_merge_ranks(alz_handle* h, int local_rc) {
   alz_comm_state* c = h->comm.get();
-  if (!c || h->comm_nranks <= 1) return ALZ_E_UNSUPPORTED;
   const int R = h->comm_nranks;
-  if (R > 64) return ALZ_E_UNSUPPORTED;
   cudaStream_t s = h->stream;
-  const unsigned grid = (unsigned)h->sms * 4;
   const uint32_t n_local = local_rc == ALZ_OK ? h->n_live : 0u;
   h->collective_bytes_last = 0;
 
@@ -470,7 +407,7 @@ int alz_internal_merge_ranks(alz_handle* h, int local_rc) {
   }
   // local rows behind the header, in canonical order; the window is NOT reset yet
   if (n_local) {
-    launch_gather_edges(h->edges, h->d_keys[1], h->d_rows[1], n_local, c->d_send + 1, false, h->sms, s);
+    launch_gather_edges(h->edges, h->d_keys, h->d_rows[1], n_local, c->d_send + 1, false, h->sms, s);
     h->launches += 1;
   }
   for (int attempt = 0; attempt < 4; ++attempt) {
@@ -479,26 +416,37 @@ int alz_internal_merge_ranks(alz_handle* h, int local_rc) {
     CK(cudaMemcpyAsync(c->d_send, c->h_hdr, sizeof(alz_edge_out), cudaMemcpyHostToDevice, s));
     const size_t block_rows = (size_t)c->cap_r + 1;
     CK(c->d_recv.ensure(block_rows * R, s));
-    CK(cudaMemsetAsync(c->d_info, 0, sizeof(MergeInfo), s));
     // the single exchange step: every rank's header + its first cap_r rows
     NK(g_nccl.AllGather(c->d_send, c->d_recv.get(), block_rows * kRowWords64, ncclUint64, c->comm, s));
     h->collective_bytes_last += (uint64_t)block_rows * R * kRowBytes;
-    merge_blocks_kernel<<<grid, 256, 0, s>>>(c->d_recv.get(), c->cap_r, (uint32_t)R, h->d_out, h->cfg.max_edges, c->d_info);
-    consume_window_kernel<<<grid, 256, 0, s>>>(c->d_info, h->edges, h->d_rows[1], n_local);
-    h->launches += 2;
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(c->h_info, c->d_info, sizeof(MergeInfo), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));   // the flush's one synchronisation: the caller needs the edge count
-    const MergeInfo inf = *c->h_info;
+    MergeInfo inf;
+    const int rc = merge_gathered(h, c, c->d_recv.get(), c->cap_r, (uint32_t)R, true, n_local, &inf);
+    if (rc != ALZ_OK) return rc;
     if (inf.peer_status != ALZ_OK) return local_rc != ALZ_OK ? local_rc : inf.peer_status;   // the window stays intact
     if (inf.overflow == 1u) { c->cap_r = block_rows_for(inf.max_count); continue; }   // every rank sees the same headers
     if (inf.overflow == 2u) return ALZ_E_CAPACITY;                                    // merged graph larger than max_edges
     c->cap_r = block_rows_for(inf.max_count);                                         // next window's block size
-    if (inf.dup) return merge_allreduce(h);                                           // not partitioned by owner: general path
-    // success: consume_window_kernel has consumed the window
-    h->last_n_edges = inf.total;
-    h->windows++;
     return ALZ_OK;
   }
   return ALZ_E_CAPACITY;
+}
+
+// test entry (alazgpu_synth.h): merge_gathered on blocks the caller gathered, with a verdict of this call's own
+extern "C" int alz_merge_blocks_device(alz_handle* h, const alz_edge_out* dev_blocks, uint32_t nranks,
+                                       uint32_t block_rows, const alz_edge_out** dev_out, size_t* n_out) {
+  if (!h || !dev_blocks || nranks < 1 || !n_out) return ALZ_E_INVAL;
+  if (nranks > kMaxRanks) return ALZ_E_UNSUPPORTED;
+  std::lock_guard<std::mutex> g(h->mu);
+  CK(cudaSetDevice(h->device));
+  *n_out = 0;
+  StatePtr<alz_comm_state> c(new alz_comm_state());
+  int rc = alloc_info(h, c.get());
+  MergeInfo inf;
+  if (rc == ALZ_OK) rc = merge_gathered(h, c.get(), dev_blocks, block_rows, nranks, false, 0, &inf);
+  if (rc != ALZ_OK) return rc;
+  if (inf.peer_status != ALZ_OK) return inf.peer_status;
+  if (inf.overflow != 0u) return ALZ_E_CAPACITY;
+  *n_out = h->last_n_edges;
+  if (dev_out) *dev_out = h->d_out;
+  return ALZ_OK;
 }

@@ -75,17 +75,6 @@ __global__ void edge_node_keys_kernel(const alz_edge_out* __restrict__ e, uint32
     out[2 * i + 1] = node_key(e[i].to_type, e[i].to);
   }
 }
-__global__ void flag_heads_kernel(const uint64_t* __restrict__ sorted, uint32_t n, uint32_t* __restrict__ flags) {
-  const uint32_t stride = gridDim.x * blockDim.x;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
-    flags[i] = (i == 0 || sorted[i - 1] != sorted[i]) ? 1u : 0u;
-}
-__global__ void scatter_heads_kernel(const uint64_t* __restrict__ sorted, const uint32_t* __restrict__ flags,
-                                     const uint32_t* __restrict__ pos, uint32_t n, uint64_t* __restrict__ out) {
-  const uint32_t stride = gridDim.x * blockDim.x;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
-    if (flags[i]) out[pos[i]] = sorted[i];
-}
 __device__ __forceinline__ uint32_t lower_bound_u64(const uint64_t* __restrict__ a, uint32_t n, uint64_t k) {
   uint32_t lo = 0, hi = n;
   while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (a[mid] < k) lo = mid + 1; else hi = mid; }
@@ -94,11 +83,6 @@ __device__ __forceinline__ uint32_t lower_bound_u64(const uint64_t* __restrict__
 
 // per node: [out_count, in_count, out_err, in_err, out_lat, in_lat, out_deg, in_deg]
 // the node count stays on the device: every consumer reads it from there, the host never waits for it
-__global__ void node_count_kernel(const uint32_t* __restrict__ pos, const uint32_t* __restrict__ flags, uint32_t n2,
-                                  uint32_t* __restrict__ n_v) {
-  if (threadIdx.x == 0 && blockIdx.x == 0) *n_v = n2 ? pos[n2 - 1] + flags[n2 - 1] : 0u;
-}
-
 __global__ void edge_stats_kernel(const alz_edge_out* __restrict__ e, uint32_t n_e, const uint64_t* __restrict__ nodes,
                                   const uint32_t* __restrict__ n_v_ptr, uint32_t* __restrict__ src_idx,
                                   uint64_t* __restrict__ dst_key, unsigned long long* __restrict__ stats,
@@ -623,10 +607,7 @@ static int gnn_run(alz_handle* h) {
   edge_node_keys_kernel<<<grid, 256, 0, s>>>(h->d_out, n_e, g->d_nk);
   launch_iota(g->d_iota, n2, h->sms, s);
   sort_pairs(g->d_tmp, g->tmp_bytes, g->d_nk, g->d_nk_sorted, g->d_iota, g->d_vals, n2, s, 34);
-  flag_heads_kernel<<<grid, 256, 0, s>>>(g->d_nk_sorted, n2, g->d_flags);
-  exclusive_scan_u32(g->d_tmp, g->tmp_bytes, g->d_flags, g->d_pos, n2, s);
-  scatter_heads_kernel<<<grid, 256, 0, s>>>(g->d_nk_sorted, g->d_flags, g->d_pos, n2, g->d_nodes);
-  node_count_kernel<<<1, 32, 0, s>>>(g->d_pos, g->d_flags, n2, g->d_nv);
+  unique_sorted_u64(g->d_tmp, g->tmp_bytes, g->d_nk_sorted, n2, g->d_flags, g->d_pos, g->d_nodes, g->d_nv, h->sms, s);
   // stats + CSR by destination (destination index < n2)
   CK(cudaMemsetAsync(g->d_stats, 0, (size_t)n2 * 64, s));
   CK(cudaMemsetAsync(g->d_in_deg, 0, ((size_t)n2 + 1) * 4, s));

@@ -180,7 +180,7 @@ struct alz_handle {
   alz::HotState* d_hot = nullptr;
 
   // flush scratch
-  uint64_t* d_keys[2] = {nullptr, nullptr};
+  uint64_t* d_keys = nullptr;             // sorted live edge keys
   uint32_t* d_rows[2] = {nullptr, nullptr};
   void* d_sort_tmp = nullptr;
   size_t sort_tmp_bytes = 0;
@@ -212,7 +212,7 @@ struct alz_handle {
 int alz_internal_fold(alz_handle* h);
 // device records -> the ingest kernel of the current mode; caller holds h->mu and has set the device
 int alz_internal_ingest(alz_handle* h, const alz_l7_rec* d_recs, size_t n);
-// multi-GPU merge of the prepared (sorted) live edges; ALZ_E_UNSUPPORTED = single rank,
-// caller finishes the flush locally. local_rc: this rank's own status so far (every rank enters the
-// collectives even when its local preparation failed, and all ranks return the same failure)
+// multi-GPU merge of the prepared (sorted) live edges, for a handle with comm_nranks > 1.
+// local_rc: this rank's own status so far (every rank enters the collective even when its local
+// preparation failed, and all ranks return the same failure)
 int alz_internal_merge_ranks(alz_handle* h, int local_rc);

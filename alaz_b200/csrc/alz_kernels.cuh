@@ -39,4 +39,8 @@ void sort_pairs(void* temp, size_t temp_bytes, const uint64_t* keys_in, uint64_t
                 const uint32_t* vals_in, uint32_t* vals_out, uint32_t n, cudaStream_t s, int end_bit = 64);
 size_t scan_temp_bytes(uint32_t n);
 void exclusive_scan_u32(void* temp, size_t temp_bytes, const uint32_t* in, uint32_t* out, uint32_t n, cudaStream_t s);
+// out[0 .. *n_unique) = the distinct values of sorted[0 .. n), ascending. The count stays on the device, so no
+// caller has to wait for it. flags and pos: n words of scratch each; temp: exclusive_scan_u32's. Three own launches.
+void unique_sorted_u64(void* temp, size_t temp_bytes, const uint64_t* sorted, uint32_t n, uint32_t* flags,
+                       uint32_t* pos, uint64_t* out, uint32_t* n_unique, int sms, cudaStream_t s);
 }  // namespace alz

@@ -245,8 +245,8 @@ int alz_submit_l7_raw(alz_handle* h, const void* host_bpf_l7_events, size_t n);
 #define ALZ_BPF_L7_EVENT_SIZE 1096
 
 /* ---- window result: the grouped rows ----------------------------------------
- * Folds pending pairs, (multi-GPU: merges all ranks, one all-reduce on the
- * accumulators), writes the live edges in ascending packed-key order
+ * Folds pending pairs, (multi-GPU: merges all ranks, one all-gather of their
+ * sorted rows), writes the live edges in ascending packed-key order
  * (docs/SPEC.md §3; the same order on every rank) and resets the window. n_out is always set to the number of live edges; if
  * cap is too small returns ALZ_E_CAPACITY and keeps the window. */
 int alz_window_flush(alz_handle* h, alz_edge_out* out, size_t cap, size_t* n_out);
@@ -340,6 +340,7 @@ int alz_sock_stats(alz_handle* h, alz_sock_stats_t* st);
 /* ---- multi-GPU: one rank per GPU, events pre-partitioned by alz_owner_rank ---- */
 #define ALZ_COMM_ID_BYTES 128
 int alz_comm_unique_id(void* out_id /* ALZ_COMM_ID_BYTES */);
+/* up to 64 ranks: ALZ_E_UNSUPPORTED for more */
 int alz_comm_init(alz_handle* h, int nranks, int rank, const void* id);
 /* rank that owns an event: hash of the source address only, so every event of
  * an edge lands on one rank before any resolve (From is the pod at saddr,

@@ -28,6 +28,13 @@ int alz_fold(alz_handle* h);
 
 /* test/debug: node keys ((kind << 32) | value, ascending) and layer-2 embeddings [n x 64] of the last GNN pass */
 int alz_gnn_nodes(alz_handle* h, uint64_t* node_keys, float* h2, size_t cap, size_t* n_out);
+/* test: the multi-rank flush's merge after its all-gather, without the collective and the window reset.
+ * dev_blocks: nranks blocks as the ranks send them, each a header row {magic, count, status} followed by
+ * block_rows rows of which `count` are live, in ascending packed-key order. The merged rows go to the handle's
+ * flush output (*dev_out, *n_out: as alz_window_flush_device). Returns a block's nonzero status, or
+ * ALZ_E_CAPACITY when a count exceeds block_rows or the rows exceed max_edges. */
+int alz_merge_blocks_device(alz_handle* h, const alz_edge_out* dev_blocks, uint32_t nranks, uint32_t block_rows,
+                            const alz_edge_out** dev_out, size_t* n_out);
 
 typedef struct alz_synth_dev alz_synth_dev;
 int alz_synth_dev_create(alz_handle* h, const alz_synth_topo* topo, alz_synth_dev** out);

@@ -47,6 +47,16 @@ def sort_edges(e):
     return e[order]
 
 
+def pack_key(e):
+    """alz_device.cuh make_edge_key on the oracle's (from,to) representation."""
+    ft, f, tt, t = int(e["from_type"]), int(e["from"]), int(e["to_type"]), int(e["to"])
+    if ft == 0:          # pod is From (canonical for pod->pod too)
+        rev, pod, ot, ov = 0, f, tt, t
+    else:                # reversed row whose From is a service / outbound host
+        rev, pod, ot, ov = 1, t, ft, f
+    return (rev << 63) | (ot << 61) | (pod << 32) | ov
+
+
 def edges_equal(a, b):
     """Bit-exact comparison of two alz_edge_out arrays (order-insensitive)."""
     a, b = sort_edges(np.asarray(a)), sort_edges(np.asarray(b))

@@ -1,6 +1,8 @@
-"""GPU, >= 2 devices: two ranks (threads, one handle per GPU) each ingest their shard, the window
-flush merges them with the single NCCL all-reduce; every rank must return the single-rank oracle's
-edges bit for bit."""
+"""GPU, >= 2 devices: the ranks (threads, one handle per GPU) each ingest their shard, the window
+flush merges them with one NCCL all-gather of their sorted rows; every rank must return the
+single-rank oracle's edges bit for bit. With overlapping shards every rank sums the rows of a key
+found on several ranks from the gathered blocks. Skips on a machine with fewer GPUs; the merge
+after the all-gather also runs on one GPU in tests/test_gpu_merge.py."""
 import ctypes as C
 import threading
 
@@ -33,7 +35,7 @@ def test_ranks_merge_to_the_single_rank_oracle(world, overlap):
     o.process(ev, 4)
     if overlap:
         # a caller that does NOT partition cleanly: the first 20k events reach every rank. The merge must
-        # notice keys present on several ranks and still return exact sums (general sort+unique path).
+        # notice keys present on several ranks and still return exact sums (sort + sum of the gathered rows).
         for _ in range(world - 1):
             o.process(ev[:20_000])
     exp = o.edges()
