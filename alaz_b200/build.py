@@ -8,7 +8,8 @@ CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIB_DIR, "libalazgpu.so")
 
-SOURCES = ["alz_api.cu", "alz_kernels.cu", "alz_ingest.cu", "alz_sort.cu", "alz_comm.cu", "alz_gnn.cu", "alz_sock.cu"]
+SOURCES = ["alz_api.cu", "alz_kernels.cu", "alz_ingest.cu", "alz_sort.cu", "alz_comm.cu", "alz_gnn.cu", "alz_sock.cu",
+           "alz_history.cu"]
 EXTRA = [os.path.join(HERE, "synth", "alz_synth_topo.c")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]

@@ -26,7 +26,7 @@ EXPORTS = [
     "alz_window_clock", "alz_window_epoch", "alz_gnn_score",
     "alz_gnn_score_device", "alz_edge_quantiles", "alz_submit_tcp", "alz_submit_tcp_raw", "alz_sock_lookup", "alz_sock_lookup_at",
     "alz_submit_l7_join", "alz_sock_gc", "alz_sock_alive", "alz_sock_stats", "alz_comm_unique_id", "alz_comm_init",
-    "alz_owner_rank",
+    "alz_owner_rank", "alz_history_init", "alz_history_info", "alz_rollup", "alz_rollup_device",
 ]
 
 
@@ -70,6 +70,10 @@ def load(rebuild=False):
         "alz_gnn_nodes": ([vp, vp, vp, sz, C.POINTER(sz)], i),
         "alz_merge_blocks_device": ([vp, vp, u32, u32, pp, C.POINTER(sz)], i),
         "alz_edge_quantiles": ([vp, vp, sz, vp], i),
+        "alz_history_init": ([vp, u32], i),
+        "alz_history_info": ([vp, C.POINTER(u32), C.POINTER(u64)], i),
+        "alz_rollup": ([vp, u32, vp, sz, C.POINTER(sz)], i),
+        "alz_rollup_device": ([vp, u32, pp, C.POINTER(sz)], i),
         "alz_submit_tcp": ([vp, vp, sz], i),
         "alz_sock_lookup": ([vp, vp, sz, vp], i),
         "alz_sock_lookup_at": ([vp, vp, sz, vp, u64], i),
@@ -239,6 +243,32 @@ class Handle:
         p = C.c_void_p()
         n = C.c_size_t(0)
         self._ck(self.L.alz_window_flush_device(self.h, C.byref(p), C.byref(n)), "alz_window_flush_device")
+        return p.value, n.value
+
+    # ---- rollups over recent windows (docs/SPEC.md §12)
+    def history_init(self, depth):
+        self._ck(self.L.alz_history_init(self.h, int(depth)), "alz_history_init")
+
+    def history_info(self):
+        """(windows held, alz_stats.windows ordinal of the newest)"""
+        held, newest = C.c_uint32(0), C.c_uint64(0)
+        self._ck(self.L.alz_history_info(self.h, C.byref(held), C.byref(newest)), "alz_history_info")
+        return held.value, newest.value
+
+    def rollup(self, k, cap=None):
+        """Rows of the sum of the newest k windows. cap=None: room for whatever the rollup returns."""
+        if cap is None:
+            p, n = self.rollup_device(k)
+            return self.d2h(p, n, abi.EDGE_OUT) if n else np.zeros(0, dtype=abi.EDGE_OUT)
+        n = C.c_size_t(0)
+        out = np.zeros(cap, dtype=abi.EDGE_OUT)
+        self._ck(self.L.alz_rollup(self.h, int(k), _ptr(out), cap, C.byref(n)), "alz_rollup")
+        return out[: n.value].copy()
+
+    def rollup_device(self, k):
+        p = C.c_void_p()
+        n = C.c_size_t(0)
+        self._ck(self.L.alz_rollup_device(self.h, int(k), C.byref(p), C.byref(n)), "alz_rollup_device")
         return p.value, n.value
 
     def stats(self):

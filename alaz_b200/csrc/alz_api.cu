@@ -656,7 +656,7 @@ static int finish_flush(alz_handle* h) {
   if (rc != ALZ_OK) return rc;
   h->last_n_edges = h->n_live;
   h->windows++;
-  return ALZ_OK;
+  return alz_internal_history_append(h);
 }
 
 // time-cut windows: the flushed epoch is closed; open the next one and submit the records that waited for it

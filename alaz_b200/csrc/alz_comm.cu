@@ -78,17 +78,6 @@ bool load_nccl() {
 
 constexpr uint32_t kMaxRanks = 64;                     // merge_blocks_kernel keeps one count per rank in shared memory
 constexpr uint32_t kRowBytes = sizeof(alz_edge_out);   // 296 = 37 x 8
-constexpr uint32_t kRowWords64 = kRowBytes / 8;
-constexpr uint32_t kSumWord = offsetof(alz_edge_out, count) / 8;   // words [kSumWord, kHistWord): u64 sums
-constexpr uint32_t kHistWord = offsetof(alz_edge_out, hist) / 8;   // words from kHistWord on: two u32 cells each
-static_assert(offsetof(alz_edge_out, lat_sum_ns) + 8 == offsetof(alz_edge_out, hist) && kHistWord * 8 ==
-              offsetof(alz_edge_out, hist), "alz_edge_out layout");
-constexpr uint32_t kHdrMagic = 0xA1A2C0DEu;
-struct BlockHeader {      // first row of a rank's block
-  uint32_t magic, count;
-  int32_t status;
-  uint32_t pad;
-};
 struct MergeInfo {        // written by the merge kernels, read by the host
   uint32_t total, dup, overflow, max_count;
   int32_t peer_status;
@@ -96,21 +85,6 @@ struct MergeInfo {        // written by the merge kernels, read by the host
   uint32_t pad[2];
 };
 
-__device__ __forceinline__ uint32_t lower_bound_u64(const uint64_t* __restrict__ a, uint32_t n, uint64_t k) {
-  uint32_t lo = 0, hi = n;
-  while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (a[mid] < k) lo = mid + 1; else hi = mid; }
-  return lo;
-}
-
-// packed edge key of an output row (inverse of unpack_edge_key)
-__device__ __forceinline__ uint64_t row_key_of(const alz_edge_out* r) {
-  // rows are 296 bytes apart: 8-byte aligned only
-  const uint2 ty = reinterpret_cast<const uint2*>(r)[0];   // from_type, to_type, pad | pad
-  const uint2 ft_ = reinterpret_cast<const uint2*>(r)[1];  // from | to
-  const uint32_t ft = ty.x & 0xFFu, tt = (ty.x >> 8) & 0xFFu;
-  if (ft == ALZ_NODE_POD) return ((uint64_t)tt << 61) | ((uint64_t)(ft_.x & 0x1FFFFFFFu) << 32) | ft_.y;
-  return (1ull << 63) | ((uint64_t)ft << 61) | ((uint64_t)(ft_.y & 0x1FFFFFFFu) << 32) | ft_.x;
-}
 __device__ __forceinline__ uint32_t lower_bound_rows(const alz_edge_out* rows, uint32_t n, uint64_t k, bool* equal) {
   uint32_t lo = 0, hi = n;
   while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (row_key_of(rows + mid) < k) lo = mid + 1; else hi = mid; }
@@ -198,55 +172,6 @@ __global__ void __launch_bounds__(256) consume_window_kernel(const MergeInfo* __
   }
 }
 
-// overlapping ranks: packed key and index in recv of every live row of the gathered blocks, in block order
-__global__ void __launch_bounds__(256) live_row_keys_kernel(const alz_edge_out* __restrict__ recv, uint32_t cap,
-                                                            uint32_t R, uint32_t total, uint64_t* __restrict__ keys,
-                                                            uint32_t* __restrict__ rows) {
-  __shared__ uint32_t s_cnt[kMaxRanks];
-  const size_t stride_rows = (size_t)cap + 1;
-  if (threadIdx.x < R) s_cnt[threadIdx.x] = reinterpret_cast<const BlockHeader*>(recv + threadIdx.x * stride_rows)->count;
-  __syncthreads();
-  const uint32_t stride = gridDim.x * blockDim.x;
-  for (uint32_t g = blockIdx.x * blockDim.x + threadIdx.x; g < total; g += stride) {
-    uint32_t q = 0, i = g;
-    while (i >= s_cnt[q]) { i -= s_cnt[q]; ++q; }
-    const uint32_t row = (uint32_t)(q * stride_rows + 1 + i);
-    keys[g] = row_key_of(recv + row);
-    rows[g] = row;
-  }
-}
-
-__device__ __forceinline__ uint64_t add_cells(uint64_t a, uint64_t b) {   // two u32 histogram cells, each modulo 2^32
-  return (uint64_t)((uint32_t)a + (uint32_t)b) | ((uint64_t)((uint32_t)(a >> 32) + (uint32_t)(b >> 32)) << 32);
-}
-
-// overlapping ranks: out[u] = the sum of the gathered rows whose key is ukeys[u]; keys/rows: all live rows, sorted
-// by key. The type and id words come from the run's first row. count, err5xx and lat_sum add modulo 2^64 and each
-// histogram cell modulo 2^32: the bits an element-wise integer sum over the ranks gives. Eight lanes per output row.
-__global__ void __launch_bounds__(256) sum_runs_kernel(const alz_edge_out* __restrict__ recv,
-                                                       const uint64_t* __restrict__ keys,
-                                                       const uint32_t* __restrict__ rows, uint32_t n,
-                                                       const uint64_t* __restrict__ ukeys,
-                                                       const uint32_t* __restrict__ n_unique,
-                                                       alz_edge_out* __restrict__ out) {
-  const uint32_t nu = *n_unique;
-  const uint32_t sl = threadIdx.x & 7u;
-  const uint32_t groups = (gridDim.x * blockDim.x) >> 3;
-  for (uint32_t u = (blockIdx.x * blockDim.x + threadIdx.x) >> 3; u < nu; u += groups) {
-    const uint64_t key = ukeys[u];
-    const uint32_t first = lower_bound_u64(keys, n, key);
-    uint64_t* d64 = reinterpret_cast<uint64_t*>(out + u);
-    for (uint32_t w = sl; w < kRowWords64; w += 8u) {
-      uint64_t v = reinterpret_cast<const uint64_t*>(recv + rows[first])[w];
-      for (uint32_t j = first + 1; w >= kSumWord && j < n && keys[j] == key; ++j) {
-        const uint64_t x = reinterpret_cast<const uint64_t*>(recv + rows[j])[w];
-        v = w < kHistWord ? v + x : add_cells(v, x);
-      }
-      d64[w] = v;
-    }
-  }
-}
-
 }  // namespace
 
 struct alz_comm_state {
@@ -261,8 +186,7 @@ struct alz_comm_state {
   BlockHeader* h_hdr = nullptr;   // pinned
   MergeInfo* d_info = nullptr;
   MergeInfo* h_info = nullptr;    // pinned
-  // overlapping ranks only, grown on first use (n = live rows of all blocks): keys [2n] (the rows' keys, then sorted;
-  // the distinct keys overwrite the first half), idx [4n] (row indices, sorted; head flags; unique positions)
+  // overlapping ranks only, grown on first use (n = live rows of all blocks): sum_blocks_by_key's scratch
   GrowBuf<uint64_t> ov_keys;
   GrowBuf<uint32_t> ov_idx;
   GrowBuf<uint8_t> ov_tmp;
@@ -334,20 +258,12 @@ extern "C" int alz_comm_init(alz_handle* h, int nranks, int rank, const void* id
 static int merge_overlap(alz_handle* h, alz_comm_state* c, const alz_edge_out* recv, uint32_t cap, uint32_t R,
                          uint32_t n, uint32_t* n_unique) {
   cudaStream_t s = h->stream;
-  const unsigned grid = (unsigned)h->sms * 4;
-  const size_t tmp_bytes = std::max(sort_pairs_temp_bytes(n), scan_temp_bytes(n));
+  const size_t tmp_bytes = sum_blocks_temp_bytes(n);
   CK(c->ov_keys.ensure(2 * (size_t)n, s));
   CK(c->ov_idx.ensure(4 * (size_t)n, s));
   CK(c->ov_tmp.ensure(tmp_bytes, s));
-  uint64_t* keys = c->ov_keys.get();
-  uint64_t* sorted = keys + n;
-  uint32_t* rows = c->ov_idx.get();
-  uint32_t* rows_sorted = rows + n;
-  live_row_keys_kernel<<<grid, 256, 0, s>>>(recv, cap, R, n, keys, rows);
-  sort_pairs(c->ov_tmp.get(), tmp_bytes, keys, sorted, rows, rows_sorted, n, s);
-  unique_sorted_u64(c->ov_tmp.get(), tmp_bytes, sorted, n, rows + 2 * (size_t)n, rows + 3 * (size_t)n, keys,
-                    &c->d_info->n_unique, h->sms, s);
-  sum_runs_kernel<<<grid, 256, 0, s>>>(recv, sorted, rows_sorted, n, keys, &c->d_info->n_unique, h->d_out);
+  sum_blocks_by_key(RowBlocks{recv, cap + 1, 0, R, R}, n, c->ov_keys.get(), c->ov_idx.get(), c->ov_tmp.get(),
+                    tmp_bytes, h->d_out, &c->d_info->n_unique, h->sms, s);
   h->launches += 5;
   CK(cudaGetLastError());
   CK(cudaMemcpyAsync(&c->h_info->n_unique, &c->d_info->n_unique, 4, cudaMemcpyDeviceToHost, s));
@@ -426,7 +342,7 @@ int alz_internal_merge_ranks(alz_handle* h, int local_rc) {
     if (inf.overflow == 1u) { c->cap_r = block_rows_for(inf.max_count); continue; }   // every rank sees the same headers
     if (inf.overflow == 2u) return ALZ_E_CAPACITY;                                    // merged graph larger than max_edges
     c->cap_r = block_rows_for(inf.max_count);                                         // next window's block size
-    return ALZ_OK;
+    return alz_internal_history_append(h);
   }
   return ALZ_E_CAPACITY;
 }

@@ -85,6 +85,15 @@ __host__ __device__ __forceinline__ void unpack_edge_key(uint64_t k, uint8_t* fr
   if (!rev) { *from_type = ALZ_NODE_POD; *from = pod; *to_type = ot; *to = other; }
   else      { *from_type = ot; *from = other; *to_type = ALZ_NODE_POD; *to = pod; }
 }
+// packed edge key of an output row (inverse of unpack_edge_key)
+__device__ __forceinline__ uint64_t row_key_of(const alz_edge_out* r) {
+  // rows are 296 bytes apart: 8-byte aligned only
+  const uint2 ty = reinterpret_cast<const uint2*>(r)[0];   // from_type, to_type, pad | pad
+  const uint2 ft_ = reinterpret_cast<const uint2*>(r)[1];  // from | to
+  const uint32_t ft = ty.x & 0xFFu, tt = (ty.x >> 8) & 0xFFu;
+  if (ft == ALZ_NODE_POD) return ((uint64_t)tt << 61) | ((uint64_t)(ft_.x & 0x1FFFFFFFu) << 32) | ft_.y;
+  return (1ull << 63) | ((uint64_t)ft << 61) | ((uint64_t)(ft_.y & 0x1FFFFFFFu) << 32) | ft_.x;
+}
 
 // ---- per-record rules ------------------------------------------------------------
 // Does processL7 hand a row to PersistRequest for this record (before resolve)?

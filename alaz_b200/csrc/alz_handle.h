@@ -117,10 +117,12 @@ static_assert(sizeof(EpPatch) == 32, "EpPatch layout");
 struct alz_gnn_state;   // alz_gnn.cu
 struct alz_sock_state;  // alz_sock.cu
 struct alz_comm_state;  // alz_comm.cu
+struct alz_history_state;   // alz_history.cu
 struct StateDelete {    // each defined beside its state
   void operator()(alz_comm_state* c) const;
   void operator()(alz_gnn_state* g) const;
   void operator()(alz_sock_state* s) const;
+  void operator()(alz_history_state* y) const;
 };
 template <class T> using StatePtr = std::unique_ptr<T, StateDelete>;
 
@@ -207,6 +209,7 @@ struct alz_handle {
   StatePtr<alz_comm_state> comm;          // optional state: published only when complete
   StatePtr<alz_gnn_state> gnn;
   StatePtr<alz_sock_state> sock;
+  StatePtr<alz_history_state> hist;       // alz_history_init
 };
 
 int alz_internal_fold(alz_handle* h);
@@ -216,3 +219,6 @@ int alz_internal_ingest(alz_handle* h, const alz_l7_rec* d_recs, size_t n);
 // local_rc: this rank's own status so far (every rank enters the collective even when its local
 // preparation failed, and all ranks return the same failure)
 int alz_internal_merge_ranks(alz_handle* h, int local_rc);
+// a flush consumed its window and counted it in h->windows: keep its rows (h->d_out, last_n_edges) in the history
+// when history is on. One device-to-device copy, no kernel; nothing at all without history.
+int alz_internal_history_append(alz_handle* h);

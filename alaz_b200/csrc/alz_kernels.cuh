@@ -43,4 +43,26 @@ void exclusive_scan_u32(void* temp, size_t temp_bytes, const uint32_t* in, uint3
 // caller has to wait for it. flags and pos: n words of scratch each; temp: exclusive_scan_u32's. Three own launches.
 void unique_sorted_u64(void* temp, size_t temp_bytes, const uint64_t* sorted, uint32_t n, uint32_t* flags,
                        uint32_t* pos, uint64_t* out, uint32_t* n_unique, int sms, cudaStream_t s);
+
+// ---- blocks of sorted edge rows: the gathered blocks of a multi-rank flush (alz_comm.cu) and the slots of the
+// window history (alz_history.cu). A block is a header row, then header.count live rows in ascending key order.
+constexpr uint32_t kRowWords64 = sizeof(alz_edge_out) / 8;   // 37
+constexpr uint32_t kHdrMagic = 0xA1A2C0DEu;
+struct BlockHeader {      // first row of a block
+  uint32_t magic, count;
+  int32_t status;
+  uint32_t pad;
+};
+// n blocks of base: block q's header is row ((first + q) % ring) * stride. Row indices are u32.
+struct RowBlocks {
+  const alz_edge_out* base;
+  uint32_t stride, first, n, ring;
+};
+// out[0 .. *n_unique) = one row per distinct packed key among the blocks' n_rows live rows, in ascending key order:
+// the type and id words of the key's first row, count, err5xx and lat_sum_ns summed modulo 2^64 and each histogram
+// cell modulo 2^32. n_rows = the sum of the header counts, > 0. keys: 2 n_rows words of scratch, idx: 4 n_rows,
+// temp: sum_blocks_temp_bytes(n_rows). The count stays on the device. Five own launches.
+size_t sum_blocks_temp_bytes(uint32_t n_rows);
+void sum_blocks_by_key(const RowBlocks& b, uint32_t n_rows, uint64_t* keys, uint32_t* idx, void* temp,
+                       size_t temp_bytes, alz_edge_out* out, uint32_t* n_unique, int sms, cudaStream_t s);
 }  // namespace alz

@@ -280,6 +280,30 @@ int alz_gnn_score_device(alz_handle* h, const float** dev_scores, size_t* n_out)
 /* quantiles from the histogram, the same float64 interpolation the scores use */
 int alz_edge_quantiles(const alz_edge_out* e, const double* qs, size_t nq, double* out_ns);
 
+/* ---- rollups over recent windows (docs/SPEC.md §12) -------------------------
+ * alz_history_init keeps the edge rows of the last `depth` flushed windows on the device, starting with the
+ * next flush. A window enters exactly when alz_stats.windows counts it: empty windows too (k windows are k
+ * clock periods), and a window that lost rows to capacity, as it was returned. A single-rank alz_window_flush
+ * that returns ALZ_E_CAPACITY before consuming the window, and a multi-rank merge larger than max_edges, do
+ * not enter. The ring, depth * (max_edges + 1) rows of 296 B, is allocated here, all or nothing; no flush
+ * allocates. ALZ_E_INVAL: depth == 0 or depth * (max_edges + 1) >= 2^32. ALZ_E_STATE: history is already on.
+ * ALZ_E_NOMEM leaves the handle without history; the call may be repeated. */
+int alz_history_init(alz_handle* h, uint32_t depth);
+/* *held: windows held (at most depth); *newest: the alz_stats.windows ordinal of the newest one (0 while none
+ * is held). With alz_window_clock, a window's epoch is its ordinal plus a fixed offset. ALZ_E_STATE without
+ * history. */
+int alz_history_info(alz_handle* h, uint32_t* held, uint64_t* newest);
+/* The sum of the newest min(k, held) windows: one row per distinct packed edge key, in ascending key order
+ * (docs/SPEC.md §3). Type and id words come from the key; count, err5xx and lat_sum_ns add modulo 2^64, each
+ * hist cell modulo 2^32. ALZ_E_INVAL: k == 0. ALZ_E_STATE: no history. held == 0 gives 0 rows. No side effects:
+ * the open window, the last flush (alz_window_fetch, alz_gnn_score), the history and the next flush are as
+ * they were. *n_out is always set; if cap is too small returns ALZ_E_CAPACITY and nothing is lost. One stream
+ * synchronisation per call. Local: no collective on a multi-rank handle, and the same bytes on every rank. */
+int alz_rollup(alz_handle* h, uint32_t k, alz_edge_out* out, size_t cap, size_t* n_out);
+/* as above but leaves the rows on the device; *dev_edges stays valid until the next alz_rollup* call on this
+ * handle */
+int alz_rollup_device(alz_handle* h, uint32_t k, const alz_edge_out** dev_edges, size_t* n_out);
+
 /* ---- tcp_state sink + temporal socket join (SURVEY §8f.2) -------------------
  * alz_submit_tcp replaces processTcpConnect (aggregator/data.go:404-506) +
  * SocketLine.AddValue (sock_num_line.go:62-80); alz_sock_lookup replaces
